@@ -123,7 +123,8 @@ class RoboyNativeError(RuntimeError):
 
 
 def lib_path():
-    # ROBOY_B200_LIB: point at another build of the same library (kernel experiments only)
+    # ROBOY_B200_LIB: load another build of the same library, e.g. another checkout's, to time two versions side by side
+    # (the compile-time kernel experiments it used to load are in commit aa5e1cc, removed afterwards)
     return os.environ.get("ROBOY_B200_LIB") or _build.LIB_PATH
 
 

@@ -47,8 +47,7 @@ def build(force=False, verbose=False):
     os.makedirs(LIB_DIR, exist_ok=True)
     obj_dir = os.path.join(os.path.dirname(_PKG), "build", "obj")
     os.makedirs(obj_dir, exist_ok=True)
-    extra = os.environ.get("ROBOY_NVCC_EXTRA", "").split()   # experiments only, e.g. -DROBOY_STEP_MIN_BLOCKS=3
-    flags = [f for f in NVCC_FLAGS if f != "-shared"] + extra + (["-Xptxas", "-v"] if verbose else [])
+    flags = [f for f in NVCC_FLAGS if f != "-shared"] + (["-Xptxas", "-v"] if verbose else [])
 
     def compile_one(src):
         obj = os.path.join(obj_dir, os.path.splitext(src)[0] + ".o")

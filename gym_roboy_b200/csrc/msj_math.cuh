@@ -107,18 +107,10 @@ struct PenaltyF32 {
 
 // sqrt of the float32 penalty sum: MUFU.SQRT directly (sqrt.approx.ftz: 2^-23 relative error, one rounding more than the
 // correctly rounded __fsqrt_rn and ~7 instructions fewer -- the penalty kernels are issue-bound: 0.909 -> 0.918 of HBM peak).
-// ROBOY_PENALTY_SQRT_APPROX=0 restores __fsqrt_rn.
-#ifndef ROBOY_PENALTY_SQRT_APPROX
-#define ROBOY_PENALTY_SQRT_APPROX 1
-#endif
 __device__ __forceinline__ float penalty_sqrt(float s) {
-#if ROBOY_PENALTY_SQRT_APPROX
     float v;
     asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(v) : "f"(s));
     return v;
-#else
-    return __fsqrt_rn(s);
-#endif
 }
 
 struct FastConsts {

@@ -243,24 +243,8 @@ namespace {
 
 // Threads per CTA of the fused step: up to 10 joints fit 128 registers (two CTAs of 256 per SM, 16 warps); beyond that a
 // thread needs ~160, and three CTAs of 128 keep 12 warps on the SM where one of 256 kept 8 (15 joints: 0.73 -> 0.76).
-#ifndef ROBOY_GENERIC_BLOCK
-#define ROBOY_GENERIC_BLOCK(JM) ((JM) <= 10 ? 256 : 128)
-#endif
-__host__ __device__ constexpr int g_step_block(int J) { return ROBOY_GENERIC_BLOCK(J); }
-#ifndef ROBOY_GENERIC_L2_PREFETCH
-#define ROBOY_GENERIC_L2_PREFETCH 1
-#endif
-#ifndef ROBOY_GENERIC_MIN_BLOCKS
-#define ROBOY_GENERIC_MIN_BLOCKS(JM) ((JM) <= 10 ? 2 : 3)   // 3 x 256 per SM spills even at one joint (measured: 0.46 vs 0.51)
-#endif
-
-// Index of joint k's constants in RobotSpec.  EXPERIMENT: -DROBOY_GENERIC_UNIFORM_PROBE reads joint 0's for every joint
-// (only right for a robot with the same bounds on every joint) to measure what a uniform-bounds instantiation would gain.
-#ifdef ROBOY_GENERIC_UNIFORM_PROBE
-#define JX(k) 0
-#else
-#define JX(k) (k)
-#endif
+__host__ __device__ constexpr int g_step_block(int J) { return J <= 10 ? 256 : 128; }
+__host__ __device__ constexpr int g_min_blocks(int J) { return J <= 10 ? 2 : 3; }   // 3 x 256 per SM spills even at one joint (measured: 0.46 vs 0.51)
 
 // value c of a state draw (see g_draw_state) with the Philox block cached across calls
 struct DrawCursor {
@@ -275,7 +259,7 @@ __device__ __forceinline__ float g_draw_value(const RobotSpec &r, const PhiloxKe
         cur.block = b;
     }
     const uint32_t k = s == 0 ? cur.d.k[0] : s == 1 ? cur.d.k[1] : s == 2 ? cur.d.k[2] : s == 3 ? cur.d.k[3] : s == 4 ? cur.d.k[4] : cur.d.k[5];
-    return uniform_in21(k, r.a_lo[JX(joint)], r.a_span21[JX(joint)]);
+    return uniform_in21(k, r.a_lo[joint], r.a_span21[joint]);
 }
 
 }  // namespace
@@ -306,7 +290,7 @@ __device__ __forceinline__ float g_mindist4(float m, const float4 &v, float c) {
 }
 
 template <int JM, bool FASTDIV>
-__global__ void __launch_bounds__(g_step_block(JM), ROBOY_GENERIC_MIN_BLOCKS(JM)) generic_step_kernel(const __grid_constant__ GStepParams p) {
+__global__ void __launch_bounds__(g_step_block(JM), g_min_blocks(JM)) generic_step_kernel(const __grid_constant__ GStepParams p) {
     constexpr int kGenericWarps = g_step_block(JM) / 32;
     extern __shared__ __align__(16) float s_stage[];          // [kGenericWarps][32 * 3J] observation rows of a chunk
     __shared__ double s_sum_reward;
@@ -334,11 +318,9 @@ __global__ void __launch_bounds__(g_step_block(JM), ROBOY_GENERIC_MIN_BLOCKS(JM)
     const bool act_vec = (A & 3) == 0 && act_al16;
     const uint32_t row_bytes = (uint32_t)A * 4;
     const int n4 = 8 * A;                                     // float4s in the 32 action rows of a full chunk
-#if ROBOY_GENERIC_L2_PREFETCH
     const char *pf_act = reinterpret_cast<const char *>(p.actions) + (size_t)lane * 128;
     // lanes 0..J-1 prefetch the line of their goal row, lane J the step words (one pointer per lane)
     const float *pf_goal = lane < J ? p.goal + (size_t)lane * n_envs : reinterpret_cast<const float *>(p.step_flags);
-#endif
     // Episode statistics cost the hot loop ONE register: the reward sum of this thread (float, like the tuned kernels; the
     // warps' sums are added in double).  Episode ends, holds and violations are rare and go to shared-memory counters
     // where they happen; the step count is the size of the range.
@@ -348,7 +330,6 @@ __global__ void __launch_bounds__(g_step_block(JM), ROBOY_GENERIC_MIN_BLOCKS(JM)
         const uint32_t e = base + lane;
         const bool live = e < e_end;
         const uint32_t rows = e_end - base < 32 ? e_end - base : 32u;
-#if ROBOY_GENERIC_L2_PREFETCH
         {   // the warp's NEXT chunk into L2 (no registers held): its action lines, one line per goal row, the step words
             const uint32_t nb = base + stride;
             if (nb + 32 <= e_end) {
@@ -358,7 +339,6 @@ __global__ void __launch_bounds__(g_step_block(JM), ROBOY_GENERIC_MIN_BLOCKS(JM)
                 if (lane <= J) asm volatile("prefetch.global.L2 [%0];" ::"l"(pf_goal + nb));
             }
         }
-#endif
 
         // ---- actions: roboy_env.py:52 assert + the hold test of simulation_client.py:38 ----
         // Fast test, whole chunk at once: the 32 rows are 32*A contiguous floats, read coalesced as float4 (a chunk starts
@@ -472,33 +452,33 @@ __global__ void __launch_bounds__(g_step_block(JM), ROBOY_GENERIC_MIN_BLOCKS(JM)
                 for (int k = 0; k < JM; ++k) {
                     const float da = __fsub_rn(q[k], g[k]);
                     est = __fmaf_rn(da, da, est);                                               // estimate of :126's sum
-                    const float tq = g_numer(q[k], r.a_hi[JX(k)], r.a_lo[JX(k)]), tg = g_numer(g[k], r.a_hi[JX(k)], r.a_lo[JX(k)]);
+                    const float tq = g_numer(q[k], r.a_hi[k], r.a_lo[k]), tg = g_numer(g[k], r.a_hi[k], r.a_lo[k]);
                     float nq, ng;
                     if (FASTDIV) {
                         g_track2(tmin, tmax, tq, tg);
-                        nq = g_div_core(tq, r.a_span[JX(k)], r.a_rcp[JX(k)]);
-                        ng = g_div_core(tg, r.a_span[JX(k)], r.a_rcp[JX(k)]);
+                        nq = g_div_core(tq, r.a_span[k], r.a_rcp[k]);
+                        ng = g_div_core(tg, r.a_span[k], r.a_rcp[k]);
                     } else {
-                        nq = __fdiv_rn(tq, r.a_span[JX(k)]);
-                        ng = __fdiv_rn(tg, r.a_span[JX(k)]);
+                        nq = __fdiv_rn(tq, r.a_span[k]);
+                        ng = __fdiv_rn(tg, r.a_span[k]);
                     }
                     const float dn = __fsub_rn(nq, ng);
                     sr = __dadd_rn(sr, (double)__fmul_rn(dn, dn));                              // compute_reward :94-96
                     if (p.penalty) {                                                            // :98-100 (float64)
-                        const float tv = g_numer(qd[k], r.v_hi[JX(k)], r.v_lo[JX(k)]);
+                        const float tv = g_numer(qd[k], r.v_hi[k], r.v_lo[k]);
                         float nv;
                         if (FASTDIV) {
                             g_track2(tmin, tmax, tv, tv);
-                            nv = g_div_core(tv, r.v_span[JX(k)], r.v_rcp[JX(k)]);
+                            nv = g_div_core(tv, r.v_span[k], r.v_rcp[k]);
                         } else {
-                            nv = __fdiv_rn(tv, r.v_span[JX(k)]);
+                            nv = __fdiv_rn(tv, r.v_span[k]);
                         }
                         if (pen32) {   // PenaltyF32 (msj_math.cuh)
-                            const float df = __fsub_rn(nv, r.v_gz_f[JX(k)]);
+                            const float df = __fsub_rn(nv, r.v_gz_f[k]);
                             spf = __fmaf_rn(df, df, spf);
                         }
                         if (pen64) {
-                            const double dp = __dsub_rn((double)nv, r.v_gz[JX(k)]);
+                            const double dp = __dsub_rn((double)nv, r.v_gz[k]);
                             sp = __fma_rn(dp, dp, sp);
                         }
                     }
@@ -528,9 +508,9 @@ __global__ void __launch_bounds__(g_step_block(JM), ROBOY_GENERIC_MIN_BLOCKS(JM)
                         } else {   // within 1e-5 of a bound of reward_range, or at the goal: the float64 sum after all
 #pragma unroll
                             for (int k = 0; k < JM; ++k) {
-                                const float tv = g_numer(qd[k], r.v_hi[JX(k)], r.v_lo[JX(k)]);
-                                const float nv = FASTDIV ? g_div_core(tv, r.v_span[JX(k)], r.v_rcp[JX(k)]) : __fdiv_rn(tv, r.v_span[JX(k)]);
-                                const double dp = __dsub_rn((double)nv, r.v_gz[JX(k)]);
+                                const float tv = g_numer(qd[k], r.v_hi[k], r.v_lo[k]);
+                                const float nv = FASTDIV ? g_div_core(tv, r.v_span[k], r.v_rcp[k]) : __fdiv_rn(tv, r.v_span[k]);
+                                const double dp = __dsub_rn((double)nv, r.v_gz[k]);
                                 sp = __fma_rn(dp, dp, sp);
                             }
                         }

@@ -28,59 +28,9 @@
 
 namespace roboy {
 
-#ifndef ROBOY_PREFETCH
-#define ROBOY_PREFETCH 1  // 0: none, 1: next chunk into registers (measured best), 2: next chunk into L2
-#endif
-
-#ifndef ROBOY_OBS_BULK_STORE
-#define ROBOY_OBS_BULK_STORE 1  // 1 (measured +1%): drain the staged observations with cp.async.bulk (TMA bulk copy smem -> global)
-#endif
-#ifndef ROBOY_HOLD_BRANCHFREE
-#define ROBOY_HOLD_BRANCHFREE 0  // 1: min/max form without a branch (measured: no gain, more spills in the open-loop kernel)
-#endif
-#ifndef ROBOY_ROLLOUT_MIN_BLOCKS
-#define ROBOY_ROLLOUT_MIN_BLOCKS ROBOY_STEP_MIN_BLOCKS
-#endif
-#ifndef ROBOY_PDL
-#define ROBOY_PDL 1  // programmatic dependent launch of the step kernel (measured: +0.7 % at 16,777,216 envs, -4 % step time at 65,536, -9 % eager at 4,096)
-#endif
-#ifndef ROBOY_DEFER_DONE
-#define ROBOY_DEFER_DONE 0  // 1: queue finished envs in shared memory and resample their goals at the end of the CTA (measured SLOWER:
-                            // 0.2606 vs 0.2563 ms per 16,777,216-env step with 1/400 of the envs finishing -- the pass is a serial tail)
-#endif
-#ifndef ROBOY_FAST_ACTION_TEST
-#define ROBOY_FAST_ACTION_TEST 1  // one NaN-propagating max-abs per float4 + warp votes; per-env ballots only when needed
-#endif
-#ifndef ROBOY_LD_HINT
-#define ROBOY_LD_HINT 0  // streamed inputs:  0 default (measured best: +3% over .cs), 1 ld.global.cs, 2 ld.global.nc.L1::no_allocate
-#endif
-#ifndef ROBOY_ST_HINT
-#define ROBOY_ST_HINT 0  // streamed outputs: 0 default, 1 st.global.cs (no measurable difference)
-#endif
-
 namespace {
 
 constexpr uint32_t kFull = 0xffffffffu;
-
-__device__ __forceinline__ float4 ld_stream(const float4 *p) {
-#if ROBOY_LD_HINT == 1
-    return __ldcs(p);
-#elif ROBOY_LD_HINT == 2
-    float4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
-#else
-    return *p;
-#endif
-}
-template <typename T>
-__device__ __forceinline__ void st_stream(T *p, const T &v) {
-#if ROBOY_ST_HINT == 1
-    __stcs(p, v);
-#else
-    *p = v;
-#endif
-}
 
 // One chunk's state inputs (32 envs): goal and step word.  The chunk's 1 KiB of actions travels separately (Actions2):
 // the actions are only ever reduced to two verdicts per env (in range? hold?).
@@ -97,18 +47,10 @@ __device__ __forceinline__ ChunkIn load_state(const StepParams &p, uint32_t base
     ChunkIn in;
     const uint32_t e = base + lane;
     if (!TAIL) {
-#ifdef ROBOY_EXPERIMENT_SKIP_GOAL
-        in.g0 = in.g1 = in.g2 = 0.25f;
-#else
         in.g0 = p.goal[e];
         in.g1 = p.goal1[e];
         in.g2 = p.goal2[e];
-#endif
-#ifdef ROBOY_EXPERIMENT_SKIP_SMALL
-        in.sf = 5u;
-#else
         in.sf = p.step_flags[e];
-#endif
     } else {  // ragged tail: out-of-range slots read as neutral values
         const uint32_t n_end = (uint32_t)p.e_end;
         const bool live = e < n_end;
@@ -126,14 +68,16 @@ struct Actions2 {
 template <bool TAIL>
 __device__ __forceinline__ Actions2 load_actions(const float *actions, uint32_t base, uint32_t n_end, int lane) {
     const float4 *a4 = reinterpret_cast<const float4 *>(actions) + (size_t)base * 2;
+    // float4(*(a4 + i)), a by-value load, compiles to the machine code the timings in DESIGN.md were taken with; plain
+    // a4[i] (nvcc 12.9) schedules the step and rollout kernels differently
     Actions2 a;
     if (!TAIL) {
-        a.a0 = ld_stream(a4 + lane);
-        a.a1 = ld_stream(a4 + 32 + lane);
+        a.a0 = float4(*(a4 + lane));
+        a.a1 = float4(*(a4 + 32 + lane));
     } else {
         const float4 z = make_float4(0.5f, 0.5f, 0.5f, 0.5f);  // ragged tail: in range, not "close to zero"
-        a.a0 = (base * 2 + lane < n_end * 2) ? ld_stream(a4 + lane) : z;
-        a.a1 = (base * 2 + 32 + lane < n_end * 2) ? ld_stream(a4 + 32 + lane) : z;
+        a.a0 = (base * 2 + lane < n_end * 2) ? float4(*(a4 + lane)) : z;
+        a.a1 = (base * 2 + 32 + lane < n_end * 2) ? float4(*(a4 + 32 + lane)) : z;
     }
     return a;
 }
@@ -155,32 +99,6 @@ __device__ __forceinline__ float maxabs4_nan(const float4 &v) {
 __device__ __forceinline__ bool action_hold4_exact(const float4 &v, float lo, float hi) {
     return v.x >= lo && v.x <= hi && v.y >= lo && v.y <= hi && v.z >= lo && v.z <= hi && v.w >= lo && v.w <= hi;
 }
-
-#if !ROBOY_FAST_ACTION_TEST   // helpers of the pre-v8 action test (kept for A/B builds)
-// roboy_env.py:52: every component inside [-1, 1] (closed; NaN fails).
-__device__ __forceinline__ bool action_ok4(const float4 &v, float hi) {
-    return fabsf(v.x) <= hi && fabsf(v.y) <= hi && fabsf(v.z) <= hi && fabsf(v.w) <= hi;
-}
-
-// simulation_client.py:38 on the rescaled action (roboy_env.py:157-158): all four components
-// inside [hold_lo, hold_hi] -- the exact pre-image of numpy's allclose(rescaled, 0), found on
-// the host by bisection over the monotone float32 map a -> rescaled(a).  Branch-free: min and max
-// of the four against the interval ends.  fminf/fmaxf drop NaNs, so the verdict is ANDed with the
-// range test of roboy_env.py:52, which is false for NaN (numpy's allclose is false for NaN too).
-#if ROBOY_HOLD_BRANCHFREE
-__device__ __forceinline__ bool action_hold4(const float4 &v, float lo, float hi, float, bool ok4) {
-    const float mn = fminf(fminf(v.x, v.y), fminf(v.z, v.w));
-    const float mx = fmaxf(fmaxf(v.x, v.y), fmaxf(v.z, v.w));
-    return ok4 && mn >= lo && mx <= hi;
-}
-#else
-__device__ __forceinline__ bool action_hold4(const float4 &v, float lo, float hi, float mag, bool) {
-    const float m = fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)));
-    if (m > mag) return false;
-    return v.x >= lo && v.x <= hi && v.y >= lo && v.y <= hi && v.z >= lo && v.z <= hi && v.w >= lo && v.w <= hi;
-}
-#endif
-#endif  // !ROBOY_FAST_ACTION_TEST
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
@@ -207,7 +125,6 @@ struct OutPtrs {
 template <bool CENTRED = true>
 __device__ __forceinline__ void test_actions(const StepParams &p, const Actions2 &act, int lane, bool live, bool &act_ok_out,
                                              bool &hold_out) {
-#if ROBOY_FAST_ACTION_TEST
     const float m_a = maxabs4_nan(act.a0), m_b = maxabs4_nan(act.a1);
     bool act_ok = true, hold = false;
     if (!CENTRED) {
@@ -236,38 +153,14 @@ __device__ __forceinline__ void test_actions(const StepParams &p, const Actions2
         const uint32_t hdm1 = __ballot_sync(kFull, m_b <= p.hold_mag && action_hold4_exact(act.a1, p.hold_lo, p.hold_hi));
         hold = live && (((lane < 16 ? hdm0 : hdm1) >> ((lane & 15) << 1)) & 3u) == 3u;
     }
-#else
-    const float hold_mag = p.hold_mag;
-    const bool ok_a = action_ok4(act.a0, p.act_in_hi), ok_b = action_ok4(act.a1, p.act_in_hi);
-    const uint32_t okm0 = __ballot_sync(kFull, ok_a);
-    const uint32_t okm1 = __ballot_sync(kFull, ok_b);
-    const uint32_t hdm0 = __ballot_sync(kFull, action_hold4(act.a0, p.hold_lo, p.hold_hi, hold_mag, ok_a));
-    const uint32_t hdm1 = __ballot_sync(kFull, action_hold4(act.a1, p.hold_lo, p.hold_hi, hold_mag, ok_b));
-    const uint32_t sh = (lane & 15) << 1;
-    const bool act_ok = (((lane < 16 ? okm0 : okm1) >> sh) & 3u) == 3u;
-    const bool hold = live && (((lane < 16 ? hdm0 : hdm1) >> sh) & 3u) == 3u;
-#endif
     act_ok_out = act_ok;
     hold_out = hold;
 }
 
-// EXPERIMENT (ROBOY_DEFER_DONE=1, not the product build): finished envs of one CTA, queued by the hot loop and worked off
-// by all threads of the CTA at its end.  An episode end costs a Philox block, three scattered goal stores and, under
-// auto-reset, a rewritten observation row: ~150 instructions that one lane of a warp executes alone, and with 1/400 of the
-// envs finishing per step 7.7 % of the 32-env chunks contain one (2.5 % of the step time at 16,777,216 envs).  Queued, the
-// instructions shrink, but the pass runs when every CTA of the persistent grid has drained its memory pipeline -- a serial
-// tail that costs more than it saves (0.2606 vs 0.2563 ms).  Entries beyond the capacity take the inline path.
-constexpr uint32_t kDoneQueueCap = 512;
-struct DoneQueue {
-    unsigned int n;
-    uint32_t env[kDoneQueueCap];   // local env id | reached << 31
-    uint32_t step[kDoneQueueCap];  // step_num at the episode end
-};
-
-template <bool PENALTY, bool BONUS, bool AUTO_RESET, int FASTDIV, bool TAIL, bool KEEP_STATE, bool DEFER = false>
+template <bool PENALTY, bool BONUS, bool AUTO_RESET, int FASTDIV, bool TAIL, bool KEEP_STATE>
 __device__ __forceinline__ uint32_t process_chunk(const StepParams &p, uint64_t t, const ChunkIn &cur, bool act_ok, bool hold,
                                                   uint32_t base, int lane, float *so, unsigned int *s_cnt, float &sum_reward,
-                                                  const OutPtrs &out, bool &done_out, DoneQueue *dq = nullptr) {
+                                                  const OutPtrs &out, bool &done_out) {
     const uint32_t e = base + lane;
     const bool live = TAIL ? (e < (uint32_t)p.e_end) : true;
 
@@ -275,12 +168,6 @@ __device__ __forceinline__ uint32_t process_chunk(const StepParams &p, uint64_t 
     const uint32_t sf = cur.sf;
     float q0, q1, q2, qd0, qd1, qd2, reward;
     bool reached, violation;
-#ifdef ROBOY_EXPERIMENT_MEMONLY  // traffic-pattern ceiling experiment: same loads/stores, no arithmetic
-    if (!hold) {
-        q0 = g0; q1 = g1; q2 = g2; qd0 = g1; qd1 = g2; qd2 = g0;
-        reward = g0 + g1; reached = false; violation = false;
-    } else
-#endif
     if (!hold) {
         // simulation_client.py:40 -> roboy_robot.py:35-39: fresh sample; velocities are drawn
         // from the ANGLE space too (reference quirk, :38)
@@ -317,22 +204,10 @@ __device__ __forceinline__ uint32_t process_chunk(const StepParams &p, uint64_t 
     row[6] = g0; row[7] = g1; row[8] = g2;
 
     if (done && live) {
-        bool queued = false;
-        if (DEFER) {
-            const unsigned int slot = atomicAdd(&dq->n, 1u);
-            if (slot < kDoneQueueCap) {
-                dq->env[slot] = e | (reached ? 0x80000000u : 0u);
-                dq->step[slot] = step;
-                if (AUTO_RESET) word = 1u | ROBOY_F_HELD_ZERO64;   // roboy_env.py:85 + the zero state of :83
-                queued = true;
-            }
-        }
-        if (!queued) {
-            // (tried: the whole warp rewriting its 128-byte goal lines instead of one lane's 4-byte partial-sector stores --
-            // 0.9404 against 0.9461 of peak in the steady state, not kept)
-            const uint32_t r = finish_episode(episode_end(p, t, e, step, reached, AUTO_RESET, row, s_cnt));
-            word = (r & 0x80000000u) ? word : (r | ROBOY_F_HELD_ZERO64);
-        }
+        // (tried: the whole warp rewriting its 128-byte goal lines instead of one lane's 4-byte partial-sector stores --
+        // 0.9404 against 0.9461 of peak in the steady state, not kept)
+        const uint32_t r = finish_episode(episode_end(p, t, e, step, reached, AUTO_RESET, row, s_cnt));
+        word = (r & 0x80000000u) ? word : (r | ROBOY_F_HELD_ZERO64);
     }
     if (live && (violation || !act_ok)) {
         atomicOr(p.err_flags, (violation ? ROBOY_ERR_REWARD_RANGE : 0u) | (!act_ok ? ROBOY_ERR_ACTION : 0u));
@@ -341,23 +216,17 @@ __device__ __forceinline__ uint32_t process_chunk(const StepParams &p, uint64_t 
     }
 
     // ---- stores ----
-#ifdef ROBOY_EXPERIMENT_SKIP_SMALL
-    if (live && reward == 123456.0f) p.step_flags[e] = word + done;
-    sum_reward += reward;
-#else
     if (live) {
         if (!KEEP_STATE) p.step_flags[e] = word;
-        st_stream(out.reward + e, reward);
+        out.reward[e] = reward;
         out.done[e] = (uint8_t)done;
         sum_reward += reward;
     }
-#endif
     done_out = done;
     if (!KEEP_STATE && p.done_bits != nullptr) {  // done mask as bits for the done-index list (uniform branch)
         const uint32_t dm = __ballot_sync(kFull, done && live);
         if (lane == 0) p.done_bits[base >> 5] = dm;
     }
-#if ROBOY_OBS_BULK_STORE
     if (!TAIL && out.obs_aligned) {
         // every lane publishes its shared-memory writes to the async proxy, then one lane hands the
         // warp's 1152 contiguous bytes to the bulk-copy engine (SASS: UBLKCP); the staging buffer is
@@ -374,14 +243,13 @@ __device__ __forceinline__ uint32_t process_chunk(const StepParams &p, uint64_t 
         }
         return word;
     }
-#endif
     __syncwarp();
     if (!TAIL && out.obs_aligned) {
         float4 *dst = reinterpret_cast<float4 *>(out.obs + (size_t)base * kObsDim);  // 1152 B per chunk: 16 B aligned
         const float4 *src = reinterpret_cast<const float4 *>(so);
-        st_stream(dst + lane, src[lane]);
-        st_stream(dst + 32 + lane, src[32 + lane]);
-        if (lane < 8) st_stream(dst + 64 + lane, src[64 + lane]);
+        dst[lane] = src[lane];
+        dst[32 + lane] = src[32 + lane];
+        if (lane < 8) dst[64 + lane] = src[64 + lane];
     } else {  // ragged tail, or a caller-supplied obs pointer that is only 4-byte aligned: scalar stores
         const uint32_t rows = TAIL ? (uint32_t)p.e_end - base : 32u;
         const uint32_t n_valid = rows * kObsDim;
@@ -395,45 +263,26 @@ __device__ __forceinline__ uint32_t process_chunk(const StepParams &p, uint64_t 
 
 template <bool PENALTY, bool BONUS, bool AUTO_RESET, int FASTDIV>
 __global__ void __launch_bounds__(kStepBlock, kStepMinBlocks) step_kernel(const __grid_constant__ StepParams p) {
-#if ROBOY_OBS_BULK_STORE
     __shared__ __align__(128) float s_obs[2][kWarpsPerBlock][32 * kObsDim];
-#else
-    __shared__ __align__(16) float s_obs[kWarpsPerBlock][32 * kObsDim];
-#endif
     __shared__ double s_red[kWarpsPerBlock];
     // rare events (done ~1/400 of env-steps, holds, violations) are counted with shared-memory
     // atomics where they happen instead of tying up registers in the hot loop
     __shared__ unsigned int s_cnt[5];  // done, success, hold, violation, sum of episode lengths
     if (threadIdx.x < 5) s_cnt[threadIdx.x] = 0;
-#if ROBOY_DEFER_DONE
-    __shared__ DoneQueue s_dq;
-    if (threadIdx.x == 0) s_dq.n = 0;
-    constexpr bool kDefer = true;
-    DoneQueue *dq = &s_dq;
-#else
-    constexpr bool kDefer = false;
-    DoneQueue *dq = nullptr;
-#endif
     __syncthreads();
-#if ROBOY_PDL
     // programmatic dependent launch: this grid may have been started while its predecessor in the stream (the policy
     // that produced the actions, or the previous step) was still draining; everything above overlapped with that.
     // From here on the predecessor's writes (actions, state, call counter) are complete and visible.
     asm volatile("griddepcontrol.wait;" ::: "memory");
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
 
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const uint64_t t = counter_begin(p.cc);
     const uint32_t n_full = (uint32_t)(p.e_end >> 5);  // chunks [chunk0, n_full) are complete
     const uint32_t warp_stride = gridDim.x * kWarpsPerBlock;
-#if ROBOY_OBS_BULK_STORE
     float *so = s_obs[0][warp];
     uint32_t parity = 0;
-#else
-    float *so = s_obs[warp];
-#endif
     // per-thread reward sum: a thread adds at most a few hundred float32 rewards per launch, the
     // cross-thread reduction below is in double
     float sum_reward = 0.0f;
@@ -460,46 +309,27 @@ __global__ void __launch_bounds__(kStepBlock, kStepMinBlocks) step_kernel(const 
         }
         bool act_ok, hold;
         test_actions<FASTDIV != kDivChecked>(p, cur_acts, lane, true, act_ok, hold);
-#if ROBOY_OBS_BULK_STORE
         // the bulk copy issued two chunks ago read this buffer: wait until at most one is still reading
         if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
         __syncwarp();
         so = s_obs[parity][warp];
         parity ^= 1;
-#endif
-        process_chunk<PENALTY, BONUS, AUTO_RESET, FASTDIV, false, false, kDefer>(p, t, cur, act_ok, hold, chunk << 5, lane, so,
-                                                                                 s_cnt, sum_reward, out, done_unused, dq);
+        process_chunk<PENALTY, BONUS, AUTO_RESET, FASTDIV, false, false>(p, t, cur, act_ok, hold, chunk << 5, lane, so, s_cnt,
+                                                                         sum_reward, out, done_unused);
         chunk = next;
     }
-#if ROBOY_OBS_BULK_STORE
-    // all bulk copies of this warp have completed (their global writes included: the queued episode ends below rewrite
-    // observation rows they wrote)
+    // all bulk copies of this warp have completed; the ragged tail below stages in buffer 0
     if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
     __syncwarp();
     so = s_obs[0][warp];
-#endif
     if (chunk == n_full && (p.e_end & 31)) {  // the ragged last chunk belongs to exactly one warp
         const Actions2 tail_acts = load_actions<true>(p.actions, chunk << 5, (uint32_t)p.e_end, lane);
         const ChunkIn cur = load_state<true>(p, chunk << 5, lane);
         bool act_ok, hold;
         test_actions<FASTDIV != kDivChecked>(p, tail_acts, lane, ((chunk << 5) + lane) < (uint32_t)p.e_end, act_ok, hold);
-        process_chunk<PENALTY, BONUS, AUTO_RESET, FASTDIV, true, false, kDefer>(p, t, cur, act_ok, hold, chunk << 5, lane, so,
-                                                                                s_cnt, sum_reward, out, done_unused, dq);
+        process_chunk<PENALTY, BONUS, AUTO_RESET, FASTDIV, true, false>(p, t, cur, act_ok, hold, chunk << 5, lane, so, s_cnt,
+                                                                        sum_reward, out, done_unused);
     }
-#if ROBOY_DEFER_DONE
-    // ---- queued episode ends: one pass of the whole CTA ----
-    __syncthreads();
-    {
-        const unsigned int qn = s_dq.n < kDoneQueueCap ? s_dq.n : kDoneQueueCap;
-        if (qn) {
-            asm volatile("fence.proxy.async;" ::: "memory");  // the rows were written through the async proxy (bulk copies)
-            for (unsigned int i = threadIdx.x; i < qn; i += kStepBlock) {
-                const uint32_t ew = s_dq.env[i];
-                finish_episode_queued(p, t, ew & 0x7fffffffu, s_dq.step[i], (ew >> 31) != 0, AUTO_RESET, out.obs, s_cnt);
-            }
-        }
-    }
-#endif
 
     // ---- K3: episode statistics, one set of atomics per CTA ----
     const double w_reward = warp_sum((double)sum_reward);
@@ -531,9 +361,6 @@ __global__ void __launch_bounds__(kStepBlock, kStepMinBlocks) step_kernel(const 
 // kNoChunk) are loaded into them, and the next chunk's goal / step-word lines are prefetched into L2 (no registers).
 // (Carrying the next chunk's state in registers as well spilled and lost 1.5 %.)
 constexpr uint32_t kNoChunk = 0xffffffffu;
-#ifndef ROBOY_ROLLOUT_L2_AHEAD
-#define ROBOY_ROLLOUT_L2_AHEAD 0   // steps of actions prefetched into L2 ahead of the register prefetch (0 / 1: off; at most 4)
-#endif
 
 template <bool PENALTY, bool BONUS, bool AUTO_RESET, int FASTDIV, bool TAIL>
 __device__ __forceinline__ void rollout_chunk(const StepParams &p, uint32_t T, uint64_t t_first, uint32_t base, int lane,
@@ -547,18 +374,8 @@ __device__ __forceinline__ void rollout_chunk(const StepParams &p, uint32_t T, u
     cur.ng1 = normalize32_hot<FASTDIV>(cur.g1, p.c.a_hi, p.c.a_lo, p.c.a_span, p.f.a_rc);
     cur.ng2 = normalize32_hot<FASTDIV>(cur.g2, p.c.a_hi, p.c.a_lo, p.c.a_span, p.f.a_rc);
     const size_t n = (size_t)p.n;
-#if ROBOY_ROLLOUT_L2_AHEAD > 1
-    // lanes 0..7 each own one of the eight 128-byte lines of a step's 32 action rows
-    const float *pf_line = p.actions + (size_t)base * kActDim + (size_t)(lane & 7) * 32;
-#endif
     for (uint32_t tt = 0; tt < T; ++tt) {
         const Actions2 cur_acts = acts;
-#if ROBOY_ROLLOUT_L2_AHEAD > 1
-        // The register prefetch below is one step deep: one memory latency per step and warp bounds the loop.  The lines
-        // of step tt + AHEAD go to L2 now (no registers), so the register load that follows AHEAD - 1 steps later is an L2 hit.
-        if (!TAIL && tt + ROBOY_ROLLOUT_L2_AHEAD < T && lane < 8)
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(pf_line + (size_t)(tt + ROBOY_ROLLOUT_L2_AHEAD) * n * kActDim));
-#endif
         if (tt + 1 < T) {
             acts = load_actions<TAIL>(p.actions + (size_t)(tt + 1) * n * kActDim, base, n_end, lane);
         } else if (!TAIL && next_base != kNoChunk) {   // hand-over to the warp's next chunk
@@ -568,21 +385,13 @@ __device__ __forceinline__ void rollout_chunk(const StepParams &p, uint32_t T, u
                                                                          : reinterpret_cast<const float *>(p.step_flags);
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(row + next_base));
             }
-#if ROBOY_ROLLOUT_L2_AHEAD > 1
-            // ... and the next chunk's steps 1 .. AHEAD - 1 (its step 0 just went into registers)
-            if (lane >= 8 && lane < 8 * ROBOY_ROLLOUT_L2_AHEAD && (uint32_t)(lane >> 3) < T)
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(p.actions + (size_t)next_base * kActDim + (size_t)(lane & 7) * 32 +
-                                                                (size_t)(lane >> 3) * n * kActDim));
-#endif
         }
         bool act_ok, hold;
         test_actions<FASTDIV != kDivChecked>(p, cur_acts, lane, live, act_ok, hold);
         const OutPtrs out{p.obs + (size_t)tt * n * kObsDim, p.reward + (size_t)tt * n, p.done + (size_t)tt * n,
                           p.obs_aligned != 0};
-#if ROBOY_OBS_BULK_STORE
         if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
         __syncwarp();
-#endif
         float *so = stage[parity][warp];
         parity ^= 1;
         bool done;
@@ -601,7 +410,7 @@ __device__ __forceinline__ void rollout_chunk(const StepParams &p, uint32_t T, u
 }
 
 template <bool PENALTY, bool BONUS, bool AUTO_RESET, int FASTDIV>
-__global__ void __launch_bounds__(kStepBlock, ROBOY_ROLLOUT_MIN_BLOCKS) rollout_kernel(const __grid_constant__ StepParams p,
+__global__ void __launch_bounds__(kStepBlock, kStepMinBlocks) rollout_kernel(const __grid_constant__ StepParams p,
                                                                             const uint32_t T) {
     __shared__ __align__(128) float s_obs[2][kWarpsPerBlock][32 * kObsDim];
     __shared__ double s_red[kWarpsPerBlock];
@@ -628,10 +437,8 @@ __global__ void __launch_bounds__(kStepBlock, ROBOY_ROLLOUT_MIN_BLOCKS) rollout_
         rollout_chunk<PENALTY, BONUS, AUTO_RESET, FASTDIV, true>(p, T, t_first, chunk << 5, lane, s_obs, warp, parity, s_cnt,
                                                                  sum_reward, acts, kNoChunk);
     }
-#if ROBOY_OBS_BULK_STORE
     if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
     __syncwarp();
-#endif
     const double w_reward = warp_sum((double)sum_reward);
     if (lane == 0) s_red[warp] = w_reward;
     __syncthreads();
@@ -741,7 +548,7 @@ cudaError_t launch_step_many(const StepParams &p, uint32_t T, bool penalty, bool
     if (!per_sm[sel]) {
         int b = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, select_rollout(sel), kStepBlock, 0) != cudaSuccess || b < 1) b = 1;
-        if (b > ROBOY_ROLLOUT_MIN_BLOCKS) b = ROBOY_ROLLOUT_MIN_BLOCKS;
+        if (b > kStepMinBlocks) b = kStepMinBlocks;
         per_sm[sel] = b;
     }
     const int grid = grid_for(p.e_end - p.e_begin, per_sm[sel], sm_count);
@@ -760,7 +567,6 @@ cudaError_t launch_step(const StepParams &p, bool penalty, bool bonus, bool auto
     if (p.e_end <= p.e_begin) return cudaSuccess;
     const int sel = selector(penalty, bonus, auto_reset, fastdiv);
     const int grid = grid_for(p.e_end - p.e_begin, blocks_per_sm(sel), sm_count);
-#if ROBOY_PDL
     static const bool pdl = [] {   // ROBOY_B200_PDL=0 in the environment turns the launch attribute off (A/B measurements)
         const char *v = getenv("ROBOY_B200_PDL");
         return !(v && v[0] == '0');
@@ -780,10 +586,6 @@ cudaError_t launch_step(const StepParams &p, bool penalty, bool bonus, bool auto
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, select_kernel(sel), p);
-#else
-    select_kernel(sel)<<<grid, kStepBlock, 0, stream>>>(p);
-    return cudaGetLastError();
-#endif
 }
 
 __global__ void counter_bump_kernel(unsigned long long *t_dev, unsigned int advance) { *t_dev += advance; }
@@ -796,10 +598,8 @@ cudaError_t launch_counter_bump(unsigned long long *t_dev, unsigned int advance,
 // Measurement only: an EMPTY kernel launched exactly like the step kernel (same grid, block, programmatic-dependent-launch
 // attribute) -- the launch floor bench.py prints next to the launch-bound sizes.
 __global__ void __launch_bounds__(kStepBlock) null_step_kernel() {
-#if ROBOY_PDL
     asm volatile("griddepcontrol.wait;" ::: "memory");
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
 }
 
 cudaError_t launch_null_step(uint64_t n_range, bool penalty, bool bonus, bool auto_reset, int fastdiv, int sm_count,
@@ -812,7 +612,7 @@ cudaError_t launch_null_step(uint64_t n_range, bool penalty, bool bonus, bool au
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = ROBOY_PDL;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, null_step_kernel);

@@ -8,15 +8,9 @@
 
 namespace roboy {
 
-#ifndef ROBOY_STEP_BLOCK
-#define ROBOY_STEP_BLOCK 256
-#endif
-constexpr int kStepBlock = ROBOY_STEP_BLOCK;  // threads per CTA of the step kernel
+constexpr int kStepBlock = 256;  // threads per CTA of the step kernel
 constexpr int kWarpsPerBlock = kStepBlock / 32;
-#ifndef ROBOY_STEP_MIN_BLOCKS
-#define ROBOY_STEP_MIN_BLOCKS 3
-#endif
-constexpr int kStepMinBlocks = ROBOY_STEP_MIN_BLOCKS;  // __launch_bounds__ min CTAs/SM (register cap)
+constexpr int kStepMinBlocks = 3;  // __launch_bounds__ min CTAs/SM (register cap)
 constexpr int kObsDim = 9, kActDim = 8;
 
 // The Philox call counter lives in device memory so that launches carry no host state and can be

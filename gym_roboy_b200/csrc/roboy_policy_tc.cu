@@ -147,38 +147,6 @@ __device__ __forceinline__ float tanh_approx(float x) {
     return y;
 }
 
-// EXPERIMENT (ROBOY_TC_FMA_TANH_EVERY > 0, not the product build): tanh WITHOUT the MUFU unit for one activation in N of
-// the fast mode -- the XU pipe (MUFU.TANH, 16 results per clock per SM) is 73 % busy while the FMA pipe idles.  Lambert's
-// continued fraction
-//   tanh x ~ x (135135 + 17325 t + 378 t^2 + t^3) / (135135 + 62370 t + 3150 t^2 + 28 t^3),   t = x^2,
-// on |x| <= 4.97 (where it reaches 1), the reciprocal from an integer-subtraction seed and two Newton steps: 16 FMA / ALU
-// instructions, abs error <= 9e-5 (tanh.approx: 5e-4 relative) -- below the float16 rounding of the result, and the GPU
-// tests pass with it.  Measured at 1,048,576 envs: N = 0 (off) 1.092e10 env-steps/s, N = 8 1.070e10, N = 6 1.070e10,
-// N = 5 9.75e9, N = 4 9.08e9 -- the 15 extra instructions per replaced tanh cost what the freed MUFU slot gains: the kernel
-// is bound by issue and latency around the MUFU unit, not by MUFU throughput alone.
-#ifndef ROBOY_TC_FMA_TANH_EVERY
-#define ROBOY_TC_FMA_TANH_EVERY 0
-#endif
-#if ROBOY_TC_FMA_TANH_EVERY > 0
-__device__ __forceinline__ float tanh_fma(float x) {
-    const float xc = fminf(fmaxf(x, -4.97f), 4.97f);
-    const float t = xc * xc;
-    const float num = xc * fmaf(t, fmaf(t, t + 378.0f, 17325.0f), 135135.0f);
-    const float den = fmaf(t, fmaf(t, fmaf(t, 28.0f, 3150.0f), 62370.0f), 135135.0f);
-    float r = __uint_as_float(0x7EF311C7u - __float_as_uint(den));
-    r = r * fmaf(-den, r, 2.0f);
-    r = r * fmaf(-den, r, 2.0f);
-    return num * r;
-}
-#endif
-// activation j of a 16-wide chunk: which unit evaluates it
-__device__ __forceinline__ float tanh_fast_mixed(float x, int j) {
-#if ROBOY_TC_FMA_TANH_EVERY > 0
-    if (j % ROBOY_TC_FMA_TANH_EVERY == ROBOY_TC_FMA_TANH_EVERY - 1) return tanh_fma(x);
-#endif
-    return tanh_approx(x);
-}
-
 struct TileCtx {
     uint32_t tmem_a;           // first column of the tile as this warp addresses it: lane quadrant in bits 31..16
     uint32_t mma_a, mma_d;     // first column of the tile / of its accumulator as the issuing thread addresses them (lane 0)
@@ -265,7 +233,7 @@ __device__ __forceinline__ void tile_activation(const TileCtx &c, const float *_
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
             if (EXACT) split_f16x2(tanh_mufu(v[2 * i]), tanh_mufu(v[2 * i + 1]), h[i], l[i]);
-            else h[i] = pack_f16x2(tanh_fast_mixed(v[2 * i], 2 * i), tanh_fast_mixed(v[2 * i + 1], 2 * i + 1));
+            else h[i] = pack_f16x2(tanh_approx(v[2 * i]), tanh_approx(v[2 * i + 1]));
         }
         tmem_st<8>(c.tmem_a + L::A + ch * 8, h);
         if (EXACT) tmem_st<8>(c.tmem_a + L::ALo + ch * 8, l);
@@ -363,7 +331,7 @@ __device__ __forceinline__ void merged_activation(const TileCtx &c) {
             tmem_ld_wait16(v);
             uint32_t h[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) h[i] = pack_f16x2(tanh_fast_mixed(v[2 * i], 2 * i), tanh_fast_mixed(v[2 * i + 1], 2 * i + 1));
+            for (int i = 0; i < 8; ++i) h[i] = pack_f16x2(tanh_approx(v[2 * i]), tanh_approx(v[2 * i + 1]));
             tmem_st<8>(c.tmem_a + (net ? M::APi : M::AVf) + ch * 8, h);
         }
     }
@@ -465,12 +433,6 @@ __global__ void __launch_bounds__(kPolicyTcMaxBlock / (MERGED ? 2 : U), 1) polic
     const float *bias32 = sd + 12;   // float32 b2 | b3 per network (exact mode)
     float sum_reward = 0.0f;
 
-#ifdef ROBOY_TC_STAGGER  // experiment: start the groups out of phase
-    {
-        const long long t0 = clock64();
-        while (clock64() - t0 < (long long)group * ROBOY_TC_STAGGER) {}
-    }
-#endif
     // all threads of a group walk the same chunks of U * 128 envs (the group's named barrier needs every one of them)
     for (uint32_t chunk = blockIdx.x * n_groups + group; chunk < n_chunks; chunk += gridDim.x * n_groups) {
         uint32_t env[U], wbase[U];   // this thread's env in tile u; first env of this warp's 32 rows of tile u

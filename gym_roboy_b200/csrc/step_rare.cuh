@@ -129,30 +129,5 @@ static __device__ __noinline__ uint32_t finish_episode(const EpisodeEnd a) {
     return 1u;                                                   // :85, with the flags replaced
 }
 
-// The same episode end, worked off after the CTA's hot loop from its shared-memory queue (closed-loop step kernel): the
-// observation row of the env is already in global memory (`obs`), so the terminal observation is copied from there and
-// the reset observation is written over it.
-static __device__ __noinline__ void finish_episode_queued(const StepParams &p, uint64_t t, uint32_t e, uint32_t step,
-                                                          bool reached, bool auto_reset, float *obs, unsigned int *s_cnt) {
-    const uint4 rg = philox_draw(p.gid_base + e, t, kStreamGoal, p.keys);
-    const float ng0 = uniform_in24(rg.x, p.c.a_lo, p.f.a_span24);
-    const float ng1 = uniform_in24(rg.y, p.c.a_lo, p.f.a_span24);
-    const float ng2 = uniform_in24(rg.z, p.c.a_lo, p.f.a_span24);
-    p.goal[e] = ng0;
-    p.goal1[e] = ng1;
-    p.goal2[e] = ng2;
-    atomicAdd(&s_cnt[0], 1u);
-    if (reached) atomicAdd(&s_cnt[1], 1u);
-    atomicAdd(&s_cnt[4], step - 1);
-    if (!auto_reset) return;
-    float *row = obs + (size_t)e * kObsDim;
-    if (p.terminal_obs) {
-#pragma unroll
-        for (int k = 0; k < kObsDim; ++k) p.terminal_obs[(size_t)e * kObsDim + k] = row[k];
-    }
-    row[0] = row[1] = row[2] = row[3] = row[4] = row[5] = 0.0f;  // reset(): zero state, :83-84,87
-    row[6] = ng0; row[7] = ng1; row[8] = ng2;
-}
-
 }  // namespace
 }  // namespace roboy
