@@ -175,7 +175,7 @@ __device__ __forceinline__ void policy_stats_tail(const StepParams &p, uint32_t 
         for (int w = 0; w < n_warps; ++w) r += s_red[w];
         const double done = (double)s_cnt[0], succ = (double)s_cnt[1];
         const double steps = blockIdx.x == 0 ? (double)(p.e_end - p.e_begin) * (double)T : 0.0;
-        const double v[ROBOY_STAT_COUNT] = {steps, done, succ, done - succ, r, (double)s_cnt[4],
+        const double v[ROBOY_STAT_COUNT] = {steps, done, succ, done - succ, r, (double)*eplen_counter(s_cnt),
                                             (double)s_cnt[2], (double)s_cnt[3]};
 #pragma unroll
         for (int k = 0; k < ROBOY_STAT_COUNT; ++k)

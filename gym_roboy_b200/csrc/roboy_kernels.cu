@@ -267,8 +267,8 @@ __global__ void __launch_bounds__(kStepBlock, kStepMinBlocks) step_kernel(const 
     __shared__ double s_red[kWarpsPerBlock];
     // rare events (done ~1/400 of env-steps, holds, violations) are counted with shared-memory
     // atomics where they happen instead of tying up registers in the hot loop
-    __shared__ unsigned int s_cnt[5];  // done, success, hold, violation, sum of episode lengths
-    if (threadIdx.x < 5) s_cnt[threadIdx.x] = 0;
+    __shared__ __align__(8) unsigned int s_cnt[kCntWords];  // done, success, hold, violation, sum of episode lengths (64-bit)
+    if (threadIdx.x < kCntWords) s_cnt[threadIdx.x] = 0;
     __syncthreads();
     // programmatic dependent launch: this grid may have been started while its predecessor in the stream (the policy
     // that produced the actions, or the previous step) was still draining; everything above overlapped with that.
@@ -341,7 +341,7 @@ __global__ void __launch_bounds__(kStepBlock, kStepMinBlocks) step_kernel(const 
         for (int w = 0; w < kWarpsPerBlock; ++w) r += s_red[w];
         const double done = (double)s_cnt[0], succ = (double)s_cnt[1];
         const double steps = blockIdx.x == 0 ? (double)(p.e_end - p.e_begin) : 0.0;
-        const double v[ROBOY_STAT_COUNT] = {steps, done, succ, done - succ, r, (double)s_cnt[4],
+        const double v[ROBOY_STAT_COUNT] = {steps, done, succ, done - succ, r, (double)*eplen_counter(s_cnt),
                                             (double)s_cnt[2], (double)s_cnt[3]};
 #pragma unroll
         for (int k = 0; k < ROBOY_STAT_COUNT; ++k)
@@ -414,8 +414,8 @@ __global__ void __launch_bounds__(kStepBlock, kStepMinBlocks) rollout_kernel(con
                                                                             const uint32_t T) {
     __shared__ __align__(128) float s_obs[2][kWarpsPerBlock][32 * kObsDim];
     __shared__ double s_red[kWarpsPerBlock];
-    __shared__ unsigned int s_cnt[5];
-    if (threadIdx.x < 5) s_cnt[threadIdx.x] = 0;
+    __shared__ __align__(8) unsigned int s_cnt[kCntWords];
+    if (threadIdx.x < kCntWords) s_cnt[threadIdx.x] = 0;
     __syncthreads();
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
@@ -448,7 +448,7 @@ __global__ void __launch_bounds__(kStepBlock, kStepMinBlocks) rollout_kernel(con
         for (int w = 0; w < kWarpsPerBlock; ++w) r += s_red[w];
         const double done = (double)s_cnt[0], succ = (double)s_cnt[1];
         const double steps = blockIdx.x == 0 ? (double)(p.e_end - p.e_begin) * (double)T : 0.0;
-        const double v[ROBOY_STAT_COUNT] = {steps, done, succ, done - succ, r, (double)s_cnt[4],
+        const double v[ROBOY_STAT_COUNT] = {steps, done, succ, done - succ, r, (double)*eplen_counter(s_cnt),
                                             (double)s_cnt[2], (double)s_cnt[3]};
 #pragma unroll
         for (int k = 0; k < ROBOY_STAT_COUNT; ++k)

@@ -142,7 +142,7 @@ __global__ void __launch_bounds__(kPolicyMaxBlock, 1) policy_rollout_kernel(cons
     unsigned int *s_cnt = reinterpret_cast<unsigned int *>(s_red + n_warps);
     for (int i = threadIdx.x; i < ROBOY_POLICY_IMAGE_FLOATS / 4; i += blockDim.x)
         reinterpret_cast<float4 *>(img)[i] = reinterpret_cast<const float4 *>(q.image)[i];
-    if (threadIdx.x < 5) s_cnt[threadIdx.x] = 0;
+    if (threadIdx.x < kCntWords) s_cnt[threadIdx.x] = 0;
     __syncthreads();
 
     const uint64_t t_first = counter_begin(p.cc);
@@ -229,7 +229,7 @@ PolicyGeom policy_geometry(uint64_t n_envs, int sm_count, int envs_per_thread) {
     if (wpb > kPolicyMaxBlock / 32) wpb = kPolicyMaxBlock / 32;
     g.block = (int)wpb * 32;
     g.smem = (int)(sizeof(float) * (ROBOY_POLICY_IMAGE_FLOATS + wpb * (kHid * 32 * g.envs_per_thread + 32 * g.envs_per_thread * kObsDim)) +
-                   sizeof(double) * wpb + sizeof(unsigned int) * 8);
+                   sizeof(double) * wpb + sizeof(unsigned int) * kCntWords);
     return g;
 }
 

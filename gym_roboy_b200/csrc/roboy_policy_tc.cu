@@ -381,13 +381,13 @@ __global__ void __launch_bounds__(kPolicyTcMaxBlock / (MERGED ? 2 : U), 1) polic
     uint64_t *mbars = reinterpret_cast<uint64_t *>(smem + kPolicyTcImagePad + n_warps * (U * 32 * kObsDim));
     double *s_red = reinterpret_cast<double *>(mbars + 4);
     unsigned int *s_cnt = reinterpret_cast<unsigned int *>(s_red + n_warps);
-    uint32_t *tmem_base_slot = s_cnt + 6;
+    uint32_t *tmem_base_slot = s_cnt + kCntWords;
     using L = Cols<EXACT>;
     // fast: the high halves of the weights and the float32 tail; exact: the whole image
     for (int i = threadIdx.x; i < ROBOY_TC_IMAGE_BYTES / 16; i += blockDim.x)
         if (EXACT || i < ROBOY_TC_OFF_LO_BYTES / 16 || i >= ROBOY_TC_OFF_STD_BYTES / 16)
             reinterpret_cast<float4 *>(img)[i] = reinterpret_cast<const float4 *>(q.image)[i];
-    if (threadIdx.x < 5) s_cnt[threadIdx.x] = 0;
+    if (threadIdx.x < kCntWords) s_cnt[threadIdx.x] = 0;
     if (threadIdx.x == 0) {
         for (int t = 0; t < n_groups * U; ++t)
             asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(smem_u32(mbars + t)) : "memory");
@@ -558,7 +558,7 @@ PolicyGeom policy_tc_geometry(uint64_t n_envs, int sm_count, int variant, bool e
     g.block = (int)groups * kTileEnvs;
     const uint64_t warps = groups * 4;
     g.smem = (int)(sizeof(float) * (kPolicyTcImagePad + warps * U * 32 * kObsDim) + 4 * sizeof(uint64_t) + sizeof(double) * warps +
-                   sizeof(unsigned int) * 8);
+                   sizeof(unsigned int) * (kCntWords + 2));   // counters, TMEM base, pad
     return g;
 }
 

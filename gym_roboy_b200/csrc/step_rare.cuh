@@ -48,6 +48,14 @@ static __device__ __noinline__ HoldOut hold_branch(const StepParams &p, uint32_t
     return o;
 }
 
+// A CTA's episode counters in shared memory, 8-byte aligned: unsigned int [0..3] episodes, successes, holds, violations;
+// [4..5] the low and high words of the 64-bit sum of episode lengths (one launch's episode ends in one CTA can add up to
+// more than 2^32 steps: 257 envs at the 2^24 - 1 cap of the step counter do), read back as one little-endian 64-bit word.
+constexpr int kCntWords = 6;
+__device__ __forceinline__ unsigned long long *eplen_counter(unsigned int *s_cnt) {
+    return reinterpret_cast<unsigned long long *>(s_cnt + 4);
+}
+
 // Everything an episode end needs, BY VALUE: the out-of-line function below must not touch the kernel's parameter block.
 // (Handed a reference to it, the compiler addressed the block generically -- 25 generic loads for the round keys and the
 // pointers plus 44 uniform-register moves, 211 instructions per call; with the values in registers and the round keys
@@ -59,7 +67,7 @@ struct EpisodeEnd {
     float *goal0, *goal1, *goal2;  // this env's slots of the goal rows
     float *terminal_row;        // this env's row of the terminal-observation side buffer, or nullptr
     float *row;                 // this env's staged observation row (shared memory)
-    unsigned int *s_cnt;
+    unsigned int *s_cnt;        // the CTA's counters (layout above)
     uint32_t step;
     uint32_t reached_auto;      // bit 0 reached, bit 1 auto_reset
 };
@@ -117,7 +125,11 @@ static __device__ __noinline__ uint32_t finish_episode(const EpisodeEnd a) {
     *a.goal2 = ng2;
     atomicAdd(&a.s_cnt[0], 1u);
     if (a.reached_auto & 1u) atomicAdd(&a.s_cnt[1], 1u);
-    atomicAdd(&a.s_cnt[4], a.step - 1);          // episode length (steps taken since reset(): step_num starts at 1)
+    // episode length (steps since reset(): step_num starts at 1) into the 64-bit counter: a 32-bit add and, when it wraps,
+    // the carry into the high word (a 64-bit atomicAdd through this generic pointer compiles to a compare-and-swap loop:
+    // 193 instructions per call against 182)
+    const uint32_t len = a.step - 1, lo = atomicAdd(&a.s_cnt[4], len);
+    if (lo + len < lo) atomicAdd(&a.s_cnt[5], 1u);
     if (!(a.reached_auto & 2u)) return a.step | 0x80000000u;  // top bit: keep the flag bits
     float *row = a.row;
     if (a.terminal_row) {

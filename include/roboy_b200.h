@@ -76,7 +76,8 @@ enum {
     ROBOY_STAT_SUCCESSES = 2,   /* ... because _did_reach_goal (roboy_env.py:125-134) */
     ROBOY_STAT_TIMEOUTS = 3,    /* ... because step_num > 400 only (roboy_env.py:72-73) */
     ROBOY_STAT_SUM_REWARD = 4,  /* sum of all step rewards */
-    ROBOY_STAT_SUM_EPLEN = 5,   /* sum of lengths of auto-reset episodes */
+    ROBOY_STAT_SUM_EPLEN = 5,   /* sum of step_num - 1 over the raised done flags (with auto_reset off, an env left done
+                                 * counts again on each further step) */
     ROBOY_STAT_HOLDS = 6,       /* steps that took the Stub's hold branch (simulation_client.py:38-39) */
     ROBOY_STAT_VIOLATIONS = 7,  /* env-steps with a non-zero error word */
     ROBOY_STAT_COUNT = 8
