@@ -112,7 +112,14 @@ def test_reward_range_bound_between_the_float32_and_the_float64_reward(robot):
         counts, firsts, rewards = [], [], []
         for f64 in (False, True):
             env, client = make(b, n, seed, True, f64)
-            client.set_reward_range(lo, float("inf"))
+            # the library re-reads ROBOY_B200_PENALTY_F64 with a new reward range: keep the float64 handle on float64
+            if f64:
+                os.environ["ROBOY_B200_PENALTY_F64"] = "1"
+            try:
+                client.set_reward_range(lo, float("inf"))
+            finally:
+                os.environ.pop("ROBOY_B200_PENALTY_F64", None)
+            assert client.penalty_float32 == (not f64)
             env.reset()
             _, r, _, _ = env.step(a)
             rewards.append(r.cpu().numpy())
