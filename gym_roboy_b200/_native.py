@@ -23,6 +23,10 @@ POLICY_HIDDEN = 64
 POLICY_OFF_W1, POLICY_OFF_B1, POLICY_OFF_W2, POLICY_OFF_B2, POLICY_OFF_W3, POLICY_OFF_B3 = 0, 576, 640, 4736, 4800, 5312
 POLICY_NET_FLOATS = 5320
 POLICY_OFF_VF, POLICY_OFF_PI, POLICY_OFF_STD, POLICY_OFF_LOGNORM, POLICY_IMAGE_FLOATS = 0, 5320, 10640, 10648, 10652
+# indices into the offsets roboy_policy_layout returns for any robot (ROBOY_POLICY_LAYOUT_*)
+(POLICY_LAYOUT_W1, POLICY_LAYOUT_B1, POLICY_LAYOUT_W2, POLICY_LAYOUT_B2, POLICY_LAYOUT_W3, POLICY_LAYOUT_VF_B3, POLICY_LAYOUT_PI_B3,
+ POLICY_LAYOUT_VF, POLICY_LAYOUT_PI, POLICY_LAYOUT_STD, POLICY_LAYOUT_LOGNORM, POLICY_LAYOUT_FLOATS) = range(12)
+POLICY_LAYOUT_WORDS = 12
 # ... and of the tensor-core variant's image (ROBOY_TC_*): float16 element offsets, then byte offsets
 TC_K_HIDDEN = 80
 TC_OFF_W1, TC_OFF_W2, TC_OFF_W3, TC_NET_HALVES, TC_OFF_VF, TC_OFF_PI = 0, 1024, 6144, 7424, 0, 7424
@@ -108,6 +112,7 @@ SIGNATURES = {
     "roboy_policy_rollout_tc": (_int, [_vp, ctypes.c_uint32, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _vp]),
     "roboy_policy_tc_geometry": (_int, [_vp, _int, _int, ctypes.POINTER(_int), ctypes.POINTER(_int), ctypes.POINTER(_int),
                                         ctypes.POINTER(_int)]),
+    "roboy_policy_layout": (_int, [_int, _int, ctypes.POINTER(ctypes.c_uint32)]),
     "roboy_policy_geometry": (_int, [_vp, _int, ctypes.POINTER(_int), ctypes.POINTER(_int), ctypes.POINTER(_int),
                                      ctypes.POINTER(_int)]),
     "roboy_launch_count": (_int, [_vp, ctypes.POINTER(_u64)]),
@@ -163,3 +168,10 @@ def dlpack_capsule(managed_tensor_ptr):
     new_capsule.restype = ctypes.py_object
     new_capsule.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p]
     return new_capsule(managed_tensor_ptr, b"dltensor", None)
+
+
+def policy_layout(dim_obs, dim_action):
+    """roboy_policy_layout: the section offsets (indexed by POLICY_LAYOUT_*) of the policy image for these dims, in floats."""
+    off = (ctypes.c_uint32 * POLICY_LAYOUT_WORDS)()
+    check(load().roboy_policy_layout(int(dim_obs), int(dim_action), off))
+    return list(off)

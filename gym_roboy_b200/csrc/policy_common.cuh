@@ -1,6 +1,7 @@
-// Pieces shared by the two fused policy rollout kernels (float32 FFMA2: roboy_policy.cu; tcgen05 TF32:
-// roboy_policy_tc.cu): the Gaussian sample, the clip and ONE env's RoboyEnv.step on the action just
-// produced -- the step kernel's arithmetic, instruction for instruction (roboy_kernels.cu, process_chunk).
+// Pieces shared by the fused policy rollout kernels (float32 FFMA2: roboy_policy.cu and, for every other robot,
+// roboy_policy_generic.cu; tcgen05 TF32: roboy_policy_tc.cu): the 64-wide dense layer, the Gaussian sample, the clip and
+// ONE env's RoboyEnv.step on the action just produced -- the MSJ step kernel's arithmetic, instruction for instruction
+// (roboy_kernels.cu, process_chunk).
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -25,6 +26,44 @@ __device__ __forceinline__ float tanh_mufu(float x) {
     return fmaf(-2.0f, r, 1.0f);
 }
 
+// acc[e][j2] (outputs 2*j2, 2*j2+1 of env e) += sum_k x_e[k] * W[k][.]; W is [K][64] in shared memory
+// (every lane reads the same 16 bytes: a broadcast), x_e[k] sits at x[k * ks + e * es] (thread-private).
+template <int E>
+__device__ __forceinline__ void dense64(const float *__restrict__ W, const float *__restrict__ x, int K, int ks, int es,
+                                        float2 (&acc)[E][32]) {
+#pragma unroll 2
+    for (int k = 0; k < K; ++k) {
+        float2 hh[E];
+#pragma unroll
+        for (int e = 0; e < E; ++e) {
+            const float h = x[k * ks + e * es];
+            hh[e] = make_float2(h, h);
+        }
+        const float4 *w4 = reinterpret_cast<const float4 *>(W + k * ROBOY_POLICY_HIDDEN);
+#pragma unroll
+        for (int jb = 0; jb < 16; ++jb) {
+            const float4 w = w4[jb];
+#pragma unroll
+            for (int e = 0; e < E; ++e) {
+                acc[e][2 * jb] = __ffma2_rn(make_float2(w.x, w.y), hh[e], acc[e][2 * jb]);
+                acc[e][2 * jb + 1] = __ffma2_rn(make_float2(w.z, w.w), hh[e], acc[e][2 * jb + 1]);
+            }
+        }
+    }
+}
+
+template <int E>
+__device__ __forceinline__ void load_bias64(const float *__restrict__ b, float2 (&acc)[E][32]) {
+#pragma unroll
+    for (int jb = 0; jb < 16; ++jb) {
+        const float4 v = reinterpret_cast<const float4 *>(b)[jb];
+#pragma unroll
+        for (int e = 0; e < E; ++e) {
+            acc[e][2 * jb] = make_float2(v.x, v.y);
+            acc[e][2 * jb + 1] = make_float2(v.z, v.w);
+        }
+    }
+}
 
 // Two standard normals from two 32-bit words (Box-Muller on the MUFU unit).
 __device__ __forceinline__ float2 box_muller(uint32_t x, uint32_t y) {
@@ -164,7 +203,9 @@ __device__ __forceinline__ void sample_and_step(const StepParams &p, const Polic
 }
 
 // Episode statistics of a launch: one set of atomics per CTA (as in step_kernel); call with all threads.
-__device__ __forceinline__ void policy_stats_tail(const StepParams &p, uint32_t T, uint64_t t_first, float sum_reward,
+// P: StepParams (the MSJ kernels) or GStepParams (the generic rollout).
+template <class P>
+__device__ __forceinline__ void policy_stats_tail(const P &p, uint32_t T, uint64_t t_first, float sum_reward,
                                                   double *s_red, unsigned int *s_cnt) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
     const double w_reward = warp_sum_d((double)sum_reward);

@@ -1374,12 +1374,34 @@ static int policy_rollout_common(roboy_env *env, bool tensor_cores, bool exact, 
     if ((uintptr_t)obs_dev & 3) return fail(ROBOY_E_ARG, "obs must be 4-byte aligned");
     if (envs_per_thread < 0 || envs_per_thread > (tensor_cores ? 3 : 2))
         return fail(ROBOY_E_ARG, "envs_per_thread must be 0, 1 or 2 (tensor-core variant: 0..3)");
-    if (!env->msj_shaped)
-        return fail(ROBOY_E_ARG, "the fused policy rollouts are built for MSJ-shaped robots (3 joints, 8 tendons, uniform bounds: "
-                                 "a 9-64-64-8 MlpPolicy); other robots step with roboy_step under a host-side policy");
+    if (!env->msj_shaped && tensor_cores)
+        return fail(ROBOY_E_ARG, "the tensor-core policy rollout is built for MSJ-shaped robots (3 joints, 8 tendons, uniform "
+                                 "bounds); other robots run the float32 rollout, roboy_policy_rollout");
+    if (!env->msj_shaped && envs_per_thread > 1)
+        return fail(ROBOY_E_ARG, "the policy rollout of robots other than MSJ runs one env per thread (envs_per_thread 0 or 1)");
     if (T == 0) return ROBOY_OK;
     DeviceGuard g(env->device);
     env->goal_sub = 1;
+    if (!env->msj_shaped) {
+        GStepParams p;
+        fill_generic_step_params(env, p, nullptr, nullptr, reward_dev, done_dev);
+        p.cc.advance = T;
+        p.done_bits = nullptr;   // the done-index list belongs to single steps
+        GPolicyParams q{};
+        q.image = image_dev;
+        if (roboy_policy_layout(env->D, env->A, q.off) != ROBOY_OK) return ROBOY_E_ARG;
+        q.T = T;
+        q.obs_aligned = (((uintptr_t)obs_dev & 15) == 0) && (env->cfg.n_envs * env->D * sizeof(float)) % 16 == 0;
+        q.obs = obs_dev;
+        q.actions = actions_dev;
+        q.logp = logp_dev;
+        q.values = values_dev;
+        q.noise = noise_dev;
+        q.noise_keys = make_philox_keys(noise_seed);
+        CUDA_TRY(launch_generic_policy_rollout(p, q, env->sm_count, (cudaStream_t)stream));
+        env->launches++;
+        return ROBOY_OK;
+    }
     StepParams p;
     fill_step_params(env, p, nullptr, obs_dev, reward_dev, done_dev);
     p.cc.advance = T;
@@ -1428,9 +1450,40 @@ int roboy_policy_tc_geometry(roboy_env *env, int tiles_per_group, int exact, int
     return ROBOY_OK;
 }
 
+int roboy_policy_layout(int dim_obs, int dim_action, uint32_t *offsets) {
+    if (!offsets) return fail(ROBOY_E_ARG, "NULL offsets");
+    if (dim_obs < 3 || dim_obs > 3 * kMaxJoint || dim_obs % 3 != 0 || dim_action < 1 || dim_action > kMaxAction)
+        return fail(ROBOY_E_ARG, "policy dims must be dim_obs = 3J with J in 1..%d and dim_action in 1..%d", kMaxJoint,
+                    kMaxAction);
+    const uint32_t D = (uint32_t)dim_obs, A8 = ((uint32_t)dim_action + 7) / 8 * 8, H = ROBOY_POLICY_HIDDEN;
+    uint32_t *o = offsets;
+    o[ROBOY_POLICY_LAYOUT_W1] = 0;
+    o[ROBOY_POLICY_LAYOUT_B1] = H * D;
+    o[ROBOY_POLICY_LAYOUT_W2] = H * D + H;
+    o[ROBOY_POLICY_LAYOUT_B2] = H * D + H + H * H;
+    o[ROBOY_POLICY_LAYOUT_W3] = H * D + 2 * H + H * H;
+    o[ROBOY_POLICY_LAYOUT_VF_B3] = o[ROBOY_POLICY_LAYOUT_W3] + H * 8;
+    o[ROBOY_POLICY_LAYOUT_PI_B3] = o[ROBOY_POLICY_LAYOUT_W3] + H * A8;
+    o[ROBOY_POLICY_LAYOUT_VF] = 0;
+    o[ROBOY_POLICY_LAYOUT_PI] = o[ROBOY_POLICY_LAYOUT_VF_B3] + 8;
+    o[ROBOY_POLICY_LAYOUT_STD] = o[ROBOY_POLICY_LAYOUT_PI] + o[ROBOY_POLICY_LAYOUT_PI_B3] + A8;
+    o[ROBOY_POLICY_LAYOUT_LOGNORM] = o[ROBOY_POLICY_LAYOUT_STD] + A8;
+    o[ROBOY_POLICY_LAYOUT_FLOATS] = (o[ROBOY_POLICY_LAYOUT_LOGNORM] + 1 + 3) / 4 * 4;
+    return ROBOY_OK;
+}
+
 int roboy_policy_geometry(roboy_env *env, int envs_per_thread, int *grid, int *block, int *smem_bytes, int *ept) {
     if (check_env(env)) return ROBOY_E_ARG;
-    const PolicyGeom geo = policy_geometry(env->cfg.n_envs, env->sm_count, envs_per_thread);
+    PolicyGeom geo;
+    if (env->msj_shaped) {
+        geo = policy_geometry(env->cfg.n_envs, env->sm_count, envs_per_thread);
+    } else {
+        if (envs_per_thread < 0 || envs_per_thread > 1)
+            return fail(ROBOY_E_ARG, "the policy rollout of robots other than MSJ runs one env per thread (envs_per_thread 0 or 1)");
+        uint32_t off[ROBOY_POLICY_LAYOUT_WORDS];
+        if (roboy_policy_layout(env->D, env->A, off) != ROBOY_OK) return ROBOY_E_ARG;
+        geo = generic_policy_geometry(env->spec.J, off[ROBOY_POLICY_LAYOUT_FLOATS], env->cfg.n_envs, env->sm_count);
+    }
     if (grid) *grid = geo.grid;
     if (block) *block = geo.block;
     if (smem_bytes) *smem_bytes = geo.smem;

@@ -38,45 +38,6 @@ namespace {
 
 constexpr int kHid = ROBOY_POLICY_HIDDEN;  // 64
 
-// acc[e][j2] (outputs 2*j2, 2*j2+1 of env e) += sum_k x_e[k] * W[k][.]; W is [K][64] in shared memory
-// (every lane reads the same 16 bytes: a broadcast), x_e[k] sits at x[k * ks + e * es] (thread-private).
-template <int E>
-__device__ __forceinline__ void dense64(const float *__restrict__ W, const float *__restrict__ x, int K, int ks, int es,
-                                        float2 (&acc)[E][32]) {
-#pragma unroll 2
-    for (int k = 0; k < K; ++k) {
-        float2 hh[E];
-#pragma unroll
-        for (int e = 0; e < E; ++e) {
-            const float h = x[k * ks + e * es];
-            hh[e] = make_float2(h, h);
-        }
-        const float4 *w4 = reinterpret_cast<const float4 *>(W + k * kHid);
-#pragma unroll
-        for (int jb = 0; jb < 16; ++jb) {
-            const float4 w = w4[jb];
-#pragma unroll
-            for (int e = 0; e < E; ++e) {
-                acc[e][2 * jb] = __ffma2_rn(make_float2(w.x, w.y), hh[e], acc[e][2 * jb]);
-                acc[e][2 * jb + 1] = __ffma2_rn(make_float2(w.z, w.w), hh[e], acc[e][2 * jb + 1]);
-            }
-        }
-    }
-}
-
-template <int E>
-__device__ __forceinline__ void load_bias64(const float *__restrict__ b, float2 (&acc)[E][32]) {
-#pragma unroll
-    for (int jb = 0; jb < 16; ++jb) {
-        const float4 v = reinterpret_cast<const float4 *>(b)[jb];
-#pragma unroll
-        for (int e = 0; e < E; ++e) {
-            acc[e][2 * jb] = make_float2(v.x, v.y);
-            acc[e][2 * jb + 1] = make_float2(v.z, v.w);
-        }
-    }
-}
-
 // One 9 -> 64 -> 64 -> 8 tanh network (the value network's output layer is zero-padded from 1 to 8
 // columns so both networks run the same code).  `row` is the envs' observation rows in the obs stage
 // (stride 9), `hs` the thread-private column of the hidden-activation scratch [64][32*E].

@@ -1,9 +1,11 @@
-// Parameter block and launcher of the fused policy rollout kernel (roboy_policy.cu).
+// Parameter blocks and launchers of the fused policy rollout kernels (roboy_policy.cu, roboy_policy_tc.cu,
+// roboy_policy_generic.cu).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include "../../include/roboy_b200.h"
+#include "roboy_generic.cuh"
 #include "roboy_kernels.cuh"
 
 namespace roboy {
@@ -42,5 +44,28 @@ cudaError_t launch_policy_rollout(const StepParams &p, const PolicyParams &q, bo
 PolicyGeom policy_tc_geometry(uint64_t n_envs, int sm_count, int tiles_per_group, bool exact);
 cudaError_t launch_policy_rollout_tc(const StepParams &p, const PolicyParams &q, bool penalty, bool bonus, bool auto_reset,
                                      bool fastdiv, int sm_count, int tiles_per_group, bool exact, cudaStream_t stream);
+
+// Float32 rollout for every robot the generic kernels take (roboy_policy_generic.cu): one env per thread, one
+// instantiation per joint count; p is as for launch_generic_step (reward / done are [T][n]; p.actions and p.obs are not
+// used), q.image is laid out by roboy_policy_layout (include/roboy_b200.h).
+constexpr int kGPolicyMaxBlock = 256;
+struct GPolicyParams {
+    const float *__restrict__ image;
+    uint32_t off[ROBOY_POLICY_LAYOUT_WORDS];   // roboy_policy_layout(3J, A)
+    uint32_t T;
+    int32_t obs_aligned;              // every obs[t] slice is 16-byte aligned
+    float *__restrict__ obs;          // [T+1][n][3J]
+    float *__restrict__ actions;      // [T][n][A]
+    float *__restrict__ logp;         // [T][n]
+    float *__restrict__ values;       // [T+1][n]
+    float *__restrict__ noise;        // [T][n][A] or nullptr
+    PhiloxKeys noise_keys;
+};
+// warps per CTA: min(8, chunks of 32 envs per SM).  The cap is kGPolicyMaxBlock / 32 = 8 (beyond 256 threads the
+// register cap makes every joint count spill).  The shared-memory budget (227 KB minus the image, per warp a 64 x 32
+// hidden column and a 32-row stage) is also applied, but never binds under that cap: 15 joints / 64 tendons, the
+// largest image, still leaves room for 11 warps.
+PolicyGeom generic_policy_geometry(int J, uint32_t image_floats, uint64_t n_envs, int sm_count);
+cudaError_t launch_generic_policy_rollout(const GStepParams &p, const GPolicyParams &q, int sm_count, cudaStream_t stream);
 
 }  // namespace roboy

@@ -1,0 +1,285 @@
+// sm_100a kernel of the closed-loop rollout for every robot the generic kernels take (J = 1..15 joints, A = 1..64
+// tendons, one bound per component): the float32 policy inside the generic env step.
+//
+// The shape is the MSJ kernel's (roboy_policy.cu): one launch runs T steps of [MlpPolicy forward -> Gaussian sample ->
+// clip -> RoboyEnv.step] for every env; a thread owns one env and keeps its observation row (shared memory), goal and
+// step word on chip for the T steps; both networks run in float32 FFMA2 with the weights broadcast from shared memory
+// (dense64, policy_common.cuh) and the hidden activations in a thread-private shared-memory column.  What changes with
+// the robot:
+//   * the first layer has D = 3J inputs; the observation stage has an ODD row stride (D rounded up to odd), so the 32
+//     lanes' reads of one input fall in 32 different banks;
+//   * the output layer has A8 = 8 * ceil(A / 8) columns.  Its 64 inputs tanh(h2) are written back into the hidden column
+//     and it runs in groups of 8 columns, each sampled, stored, clipped and action-tested before the next, so no more
+//     than 8 outputs are ever in registers.  Every output is b3 + sum_j tanh(h2_j) * W3[j] with j ascending, the
+//     operation order of the MSJ kernel: for MSJ the two give the same bits;
+//   * normal k (k < A) is Box-Muller on word pair (k mod 4) / 2 of Philox block (stream 4, sub = k / 4) keyed by the
+//     noise seed, the first or second value by k mod 2 -- for A = 8 exactly the MSJ kernel's draws;
+//   * the env step is generic_env_step (generic_env.cuh), the per-env body of generic_step_kernel: given the clipped
+//     actions this kernel stores, T roboy_step calls reproduce its env outputs bit for bit.
+// Per env-step the kernel writes actions 4A + logp 4 + value 4 + obs 12J + reward 4 + done 1 = 4A + 12J + 13 bytes and
+// evaluates 64 * (2D + 128 + 8 + A8) FMAs.
+#include <cuda_runtime.h>
+#include <math.h>
+
+#include "../../include/roboy_b200.h"
+#include "generic_env.cuh"
+#include "policy_common.cuh"
+#include "roboy_generic.cuh"
+#include "roboy_policy.cuh"
+
+namespace roboy {
+
+namespace {
+
+constexpr int kGHid = ROBOY_POLICY_HIDDEN;  // 64
+constexpr int kGPolicySmemBudget = 227 * 1024;
+
+// tanh(h2) of one network into the thread's hidden column hs[j * 32] (j = 0..63); `row` is the env's observation row
+template <int D>
+__device__ __forceinline__ void mlp_hidden(const float *__restrict__ net, const uint32_t (&off)[ROBOY_POLICY_LAYOUT_WORDS],
+                                           const float *__restrict__ row, float *__restrict__ hs) {
+    float2 acc[1][32];
+    load_bias64<1>(net + off[ROBOY_POLICY_LAYOUT_B1], acc);
+    dense64<1>(net + off[ROBOY_POLICY_LAYOUT_W1], row, D, 1, 0, acc);
+#pragma unroll
+    for (int j2 = 0; j2 < 32; ++j2) {
+        hs[(2 * j2) * 32] = tanh_mufu(acc[0][j2].x);
+        hs[(2 * j2 + 1) * 32] = tanh_mufu(acc[0][j2].y);
+    }
+    load_bias64<1>(net + off[ROBOY_POLICY_LAYOUT_B2], acc);
+    dense64<1>(net + off[ROBOY_POLICY_LAYOUT_W2], hs, kGHid, 32, 0, acc);
+#pragma unroll
+    for (int j2 = 0; j2 < 32; ++j2) {
+        hs[(2 * j2) * 32] = tanh_mufu(acc[0][j2].x);
+        hs[(2 * j2 + 1) * 32] = tanh_mufu(acc[0][j2].y);
+    }
+}
+
+// Output columns 8c .. 8c + 7 of the last layer: b3 + sum_j tanh(h2_j) * W3[j] (W3 is [64][W], b3 [W])
+__device__ __forceinline__ void mlp_out8(const float *__restrict__ w3, const float *__restrict__ b3, int W, int c,
+                                         const float *__restrict__ hs, float (&out)[8]) {
+    const float4 b0 = reinterpret_cast<const float4 *>(b3 + 8 * c)[0];
+    const float4 b1 = reinterpret_cast<const float4 *>(b3 + 8 * c)[1];
+    float2 o[4] = {make_float2(b0.x, b0.y), make_float2(b0.z, b0.w), make_float2(b1.x, b1.y), make_float2(b1.z, b1.w)};
+    const float *w = w3 + 8 * c;
+#pragma unroll 8
+    for (int j = 0; j < kGHid; ++j) {
+        const float4 wa = reinterpret_cast<const float4 *>(w + j * W)[0], wb = reinterpret_cast<const float4 *>(w + j * W)[1];
+        const float t = hs[j * 32];
+        const float2 tt = make_float2(t, t);
+        o[0] = __ffma2_rn(make_float2(wa.x, wa.y), tt, o[0]);
+        o[1] = __ffma2_rn(make_float2(wa.z, wa.w), tt, o[1]);
+        o[2] = __ffma2_rn(make_float2(wb.x, wb.y), tt, o[2]);
+        o[3] = __ffma2_rn(make_float2(wb.z, wb.w), tt, o[3]);
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        out[2 * k] = o[k].x;
+        out[2 * k + 1] = o[k].y;
+    }
+}
+
+__host__ __device__ constexpr int g_stage_stride(int J) { return (3 * J) | 1; }
+
+}  // namespace
+
+template <int JM>
+__global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_rollout_kernel(const __grid_constant__ GStepParams p,
+                                                                                      const __grid_constant__ GPolicyParams q) {
+    constexpr int J = JM, D = 3 * J, S = g_stage_stride(J);
+    const RobotSpec &r = p.r;
+    const int A = r.A, A8 = (A + 7) & ~7;
+    extern __shared__ __align__(16) float smem[];
+    const int lane = threadIdx.x & 31;
+    const int warp = threadIdx.x >> 5;
+    const int n_warps = blockDim.x >> 5;
+    // shared memory: policy image | per warp: hidden column [64][32] | obs stage [32][S] | reduction | counters
+    const uint32_t img_floats = q.off[ROBOY_POLICY_LAYOUT_FLOATS];
+    float *img = smem;
+    float *hs = smem + img_floats + warp * (kGHid * 32) + lane;
+    float *stage = smem + img_floats + n_warps * (kGHid * 32) + warp * (32 * S);
+    double *s_red = reinterpret_cast<double *>(smem + img_floats + n_warps * (kGHid * 32 + 32 * S));
+    unsigned int *s_cnt = reinterpret_cast<unsigned int *>(s_red + n_warps);
+    for (uint32_t i = threadIdx.x; i < img_floats / 4; i += blockDim.x)
+        reinterpret_cast<float4 *>(img)[i] = reinterpret_cast<const float4 *>(q.image)[i];
+    if (threadIdx.x < kCntWords) s_cnt[threadIdx.x] = 0;
+    __syncthreads();
+
+    const uint64_t t_first = counter_begin(p.cc);
+    const uint32_t n_end = (uint32_t)p.e_end, n_envs = (uint32_t)p.n;
+    const size_t n = (size_t)p.n;
+    const uint32_t n_chunks = (n_end + 31) / 32;
+    const uint32_t warp_stride = gridDim.x * n_warps;
+    const float *vf_net = img + q.off[ROBOY_POLICY_LAYOUT_VF], *pi_net = img + q.off[ROBOY_POLICY_LAYOUT_PI];
+    const float *sd = img + q.off[ROBOY_POLICY_LAYOUT_STD];
+    const float lognorm = img[q.off[ROBOY_POLICY_LAYOUT_LOGNORM]];
+    const bool fastdiv = r.fastdiv != 0;   // the step kernel's choice (launch_generic_step)
+    const bool act_vec = (A & 3) == 0;   // rows of actions / noise are 16-byte aligned (the buffers are)
+    float *row = stage + lane * S;
+    float sum_reward = 0.0f;
+
+    for (uint32_t chunk = blockIdx.x * n_warps + warp; chunk < n_chunks; chunk += warp_stride) {
+        const uint32_t base = chunk * 32;
+        const bool full = base + 32 <= n_end;
+        const uint32_t env = base + lane;
+        const bool live = env < n_end;
+        const uint64_t gid = p.gid_base + env;
+        float g[JM];
+        uint32_t sf = live ? p.step_flags[env] : 0u;
+#pragma unroll
+        for (int k = 0; k < JM; ++k) g[k] = live ? p.goal[(size_t)k * n + env] : 0.f;
+        __syncwarp();
+        // the observation the rollout starts from: slot 0 of the obs buffer
+#pragma unroll
+        for (int k = 0; k < D; ++k) row[k] = live ? q.obs[(size_t)env * D + k] : 0.f;
+
+        for (uint32_t tt = 0;; ++tt) {
+            // ---- value network on obs[tt] (also the bootstrap value at tt == T) ----
+            mlp_hidden<D>(vf_net, q.off, row, hs);
+            {
+                float v[8];
+                mlp_out8(vf_net + q.off[ROBOY_POLICY_LAYOUT_W3], vf_net + q.off[ROBOY_POLICY_LAYOUT_VF_B3], 8, 0, hs, v);
+                if (live) q.values[(size_t)tt * n + env] = v[0];
+            }
+            if (tt == q.T) break;
+            // ---- policy network, 8 output columns at a time: mean -> a = mean + std * z -> clip -> action tests ----
+            mlp_hidden<D>(pi_net, q.off, row, hs);
+            const uint64_t t = t_first + tt;
+            const size_t slot = (size_t)tt * n + env;
+            float zz = 0.0f;
+            bool act_ok = true, hold = live;
+            for (int c = 0; c < A8 / 8; ++c) {
+                float mean[8];
+                mlp_out8(pi_net + q.off[ROBOY_POLICY_LAYOUT_W3], pi_net + q.off[ROBOY_POLICY_LAYOUT_PI_B3], A8, c, hs, mean);
+                const uint4 r0 = philox_draw(gid, t, kStreamNoise, q.noise_keys, 2 * c);
+                const uint4 r1 = philox_draw(gid, t, kStreamNoise, q.noise_keys, 2 * c + 1);
+                const float2 z01 = box_muller(r0.x, r0.y), z23 = box_muller(r0.z, r0.w);
+                const float2 z45 = box_muller(r1.x, r1.y), z67 = box_muller(r1.z, r1.w);
+                const float z[8] = {z01.x, z01.y, z23.x, z23.y, z45.x, z45.y, z67.x, z67.y};
+                float u[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const int k = 8 * c + i;
+                    u[i] = fmaf(sd[k], z[i], mean[i]);
+                    if (k < A) {
+                        const float cl = fminf(fmaxf(u[i], -1.0f), 1.0f);
+                        const float a = (u[i] != u[i]) ? u[i] : cl;   // a NaN stays a NaN (and fails the assert)
+                        zz = fmaf(z[i], z[i], zz);
+                        act_ok = act_ok && (a >= -1.0f && a <= 1.0f);                      // roboy_env.py:52
+                        hold = hold && (a >= r.hold_lo[k] && a <= r.hold_hi[k]);           // simulation_client.py:38
+                    }
+                }
+                if (live) {
+                    float *ap = q.actions + slot * A + 8 * c;
+                    float *np = q.noise ? q.noise + slot * A + 8 * c : nullptr;
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        if (act_vec) {
+                            if (8 * c + 4 * h < A) {
+                                reinterpret_cast<float4 *>(ap)[h] = make_float4(u[4 * h], u[4 * h + 1], u[4 * h + 2], u[4 * h + 3]);
+                                if (np) reinterpret_cast<float4 *>(np)[h] = make_float4(z[4 * h], z[4 * h + 1], z[4 * h + 2], z[4 * h + 3]);
+                            }
+                        } else {
+#pragma unroll
+                            for (int i = 4 * h; i < 4 * h + 4; ++i)
+                                if (8 * c + i < A) {
+                                    ap[i] = u[i];
+                                    if (np) np[i] = z[i];
+                                }
+                        }
+                    }
+                }
+            }
+            if (live) q.logp[slot] = fmaf(-0.5f, zz, lognorm);
+
+            // ---- RoboyEnv.step on the clipped action: the generic step kernel's per-env body ----
+            float qs[JM], qds[JM];
+#pragma unroll
+            for (int k = 0; k < JM; ++k) qs[k] = qds[k] = 0.0f;
+            if (live) {
+                DrawCursor cur;
+                cur.block = 0xffffffffu;
+#pragma unroll
+                for (int k = 0; k < JM; ++k) qs[k] = g_draw_value(r, p.keys, gid, t, cur, k, k);
+#pragma unroll
+                for (int k = 0; k < JM; ++k) qds[k] = g_draw_value(r, p.keys, gid, t, cur, J + k, k);
+            }
+            const bool done = generic_env_step<JM>(p, fastdiv, live, hold, act_ok, qs, qds, g, sf, gid, t, env, n_envs, s_cnt,
+                                                   eplen_counter(s_cnt), sum_reward, [&](uint32_t word, float rf, bool d) {
+                                                       sf = word;
+                                                       p.reward[slot] = rf;
+                                                       p.done[slot] = (uint8_t)d;
+                                                   });
+            // ---- obs[tt + 1] = [q, qd, goal] into the stage, then the chunk's 32 rows out coalesced ----
+#pragma unroll
+            for (int k = 0; k < JM; ++k) {
+                row[k] = qs[k];
+                row[J + k] = qds[k];
+                row[2 * J + k] = g[k];
+            }
+            if (done) {   // the goal of the next step (done without auto-reset: the observation above shows the old one)
+#pragma unroll
+                for (int k = 0; k < JM; ++k) g[k] = p.goal[(size_t)k * n + env];
+            }
+            __syncwarp();
+            float *dst = q.obs + ((size_t)(tt + 1) * n + base) * D;
+            if (full && q.obs_aligned) {   // 32 rows = 8D float4s
+                float4 *dst4 = reinterpret_cast<float4 *>(dst);
+                for (int i4 = lane; i4 < 8 * D; i4 += 32) {
+                    float v[4];
+#pragma unroll
+                    for (int c = 0; c < 4; ++c) {
+                        const int i = 4 * i4 + c;
+                        v[c] = stage[(i / D) * S + i % D];
+                    }
+                    dst4[i4] = make_float4(v[0], v[1], v[2], v[3]);
+                }
+            } else {
+                const uint32_t rows = full ? 32u : n_end - base;
+                for (uint32_t i = lane; i < rows * D; i += 32) dst[i] = stage[(i / D) * S + i % D];
+            }
+            __syncwarp();
+        }
+        if (live) p.step_flags[env] = sf;
+    }
+
+    policy_stats_tail(p, q.T, t_first, sum_reward, s_red, s_cnt);
+}
+
+PolicyGeom generic_policy_geometry(int J, uint32_t image_floats, uint64_t n_envs, int sm_count) {
+    PolicyGeom g;
+    g.envs_per_thread = 1;
+    const int per_warp = (int)sizeof(float) * (kGHid * 32 + 32 * g_stage_stride(J)) + (int)sizeof(double);
+    const int fixed = (int)sizeof(float) * (int)image_floats + (int)sizeof(unsigned int) * kCntWords;
+    int max_warps = (kGPolicySmemBudget - fixed) / per_warp;
+    if (max_warps > kGPolicyMaxBlock / 32) max_warps = kGPolicyMaxBlock / 32;
+    const uint64_t n_chunks = (n_envs + 31) / 32;
+    // spread the warps over the SMs first, then fill the CTAs (one CTA per SM)
+    g.grid = (int)(n_chunks < (uint64_t)sm_count ? n_chunks : (uint64_t)sm_count);
+    uint64_t wpb = (n_chunks + g.grid - 1) / g.grid;
+    if (wpb > (uint64_t)max_warps) wpb = (uint64_t)max_warps;
+    g.block = (int)wpb * 32;
+    g.smem = fixed + (int)wpb * per_warp;
+    return g;
+}
+
+cudaError_t launch_generic_policy_rollout(const GStepParams &p, const GPolicyParams &q, int sm_count, cudaStream_t stream) {
+    if (p.e_end <= p.e_begin) return cudaSuccess;
+    const PolicyGeom g = generic_policy_geometry(p.r.J, q.off[ROBOY_POLICY_LAYOUT_FLOATS], p.e_end, sm_count);
+    void (*fn)(const GStepParams, const GPolicyParams) = nullptr;
+    switch (p.r.J) {
+#define ROBOY_GPOLICY_CASE(JJ) \
+        case JJ: fn = generic_policy_rollout_kernel<JJ>; break;
+        ROBOY_GPOLICY_CASE(1) ROBOY_GPOLICY_CASE(2) ROBOY_GPOLICY_CASE(3) ROBOY_GPOLICY_CASE(4) ROBOY_GPOLICY_CASE(5)
+        ROBOY_GPOLICY_CASE(6) ROBOY_GPOLICY_CASE(7) ROBOY_GPOLICY_CASE(8) ROBOY_GPOLICY_CASE(9) ROBOY_GPOLICY_CASE(10)
+        ROBOY_GPOLICY_CASE(11) ROBOY_GPOLICY_CASE(12) ROBOY_GPOLICY_CASE(13) ROBOY_GPOLICY_CASE(14) ROBOY_GPOLICY_CASE(15)
+#undef ROBOY_GPOLICY_CASE
+        default: return cudaErrorInvalidValue;
+    }
+    cudaError_t err = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem);
+    if (err != cudaSuccess) return err;
+    fn<<<g.grid, g.block, g.smem, stream>>>(p, q);
+    return cudaGetLastError();
+}
+
+}  // namespace roboy

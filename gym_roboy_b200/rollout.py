@@ -56,30 +56,42 @@ def gae(rewards, values, dones, last_value, gamma=0.99, lam=0.95, adv=None, ret=
 
 
 def pack_policy_image(policy, out=None):
-    """Pack an `MlpPolicy` into the float32 image `roboy_policy_rollout` reads (layout: ROBOY_POLICY_* in
-    include/roboy_b200.h): per network W1^T | b1 | W2^T | b2 | W3^T (8 columns) | b3 (8), value network first,
-    then std = exp(log_std) and the log-density constant."""
+    """Pack an `MlpPolicy(obs_dim=3J, act_dim=A)` into the float32 image `roboy_policy_rollout` reads, at the offsets
+    `roboy_policy_layout` gives (include/roboy_b200.h): per network W1^T | b1 | W2^T | b2 | W3^T | b3 with the output
+    columns zero-padded to 8 (value) or to a multiple of 8 (policy), value network first, then std = exp(log_std)
+    and the log-density constant.  For MSJ (9, 8) that is the ROBOY_POLICY_OFF_* image."""
     N = _native
     dev = policy.log_std.device
-    img = torch.zeros(N.POLICY_IMAGE_FLOATS, dtype=torch.float32, device=dev) if out is None else out
-    for base, net in ((N.POLICY_OFF_VF, policy.vf), (N.POLICY_OFF_PI, policy.pi)):
+    l1 = policy.pi[0]
+    d_obs, d_act = l1.weight.shape[1], policy.log_std.numel()
+    off = N.policy_layout(d_obs, d_act)
+    a8 = (d_act + 7) // 8 * 8
+    H = N.POLICY_HIDDEN
+    img = torch.zeros(off[N.POLICY_LAYOUT_FLOATS], dtype=torch.float32, device=dev) if out is None else out
+    assert img.numel() == off[N.POLICY_LAYOUT_FLOATS] and img.dtype == torch.float32
+    for base, net, n_out, cols, b3_at in ((off[N.POLICY_LAYOUT_VF], policy.vf, 1, 8, off[N.POLICY_LAYOUT_VF_B3]),
+                                          (off[N.POLICY_LAYOUT_PI], policy.pi, d_act, a8, off[N.POLICY_LAYOUT_PI_B3])):
         l1, l2, l3 = net[0], net[2], net[4]
-        assert l1.weight.shape == (N.POLICY_HIDDEN, N.DIM_OBS) and l2.weight.shape == (N.POLICY_HIDDEN, N.POLICY_HIDDEN)
-        n_out = l3.weight.shape[0]
-        assert n_out in (1, N.DIM_ACTION)
-        img[base + N.POLICY_OFF_W1: base + N.POLICY_OFF_B1].copy_(l1.weight.detach().t().reshape(-1))
-        img[base + N.POLICY_OFF_B1: base + N.POLICY_OFF_W2].copy_(l1.bias.detach())
-        img[base + N.POLICY_OFF_W2: base + N.POLICY_OFF_B2].copy_(l2.weight.detach().t().reshape(-1))
-        img[base + N.POLICY_OFF_B2: base + N.POLICY_OFF_W3].copy_(l2.bias.detach())
-        w3 = img[base + N.POLICY_OFF_W3: base + N.POLICY_OFF_B3].view(N.POLICY_HIDDEN, 8)
-        w3.zero_()
-        w3[:, :n_out].copy_(l3.weight.detach().t())
-        b3 = img[base + N.POLICY_OFF_B3: base + N.POLICY_NET_FLOATS]
-        b3.zero_()
-        b3[:n_out].copy_(l3.bias.detach())
+        assert l1.weight.shape == (H, d_obs) and l2.weight.shape == (H, H) and l3.weight.shape == (n_out, H)
+        w1, b1, w2, b2, w3 = (base + off[k] for k in (N.POLICY_LAYOUT_W1, N.POLICY_LAYOUT_B1, N.POLICY_LAYOUT_W2,
+                                                       N.POLICY_LAYOUT_B2, N.POLICY_LAYOUT_W3))
+        b3 = base + b3_at
+        img[w1:b1].copy_(l1.weight.detach().t().reshape(-1))
+        img[b1:w2].copy_(l1.bias.detach())
+        img[w2:b2].copy_(l2.weight.detach().t().reshape(-1))
+        img[b2:w3].copy_(l2.bias.detach())
+        w3v = img[w3:b3].view(H, cols)
+        w3v.zero_()
+        w3v[:, :n_out].copy_(l3.weight.detach().t())
+        b3v = img[b3:b3 + cols]
+        b3v.zero_()
+        b3v[:n_out].copy_(l3.bias.detach())
     log_std = policy.log_std.detach()
-    img[N.POLICY_OFF_STD: N.POLICY_OFF_STD + 8].copy_(log_std.exp())
-    img[N.POLICY_OFF_LOGNORM] = -0.5 * math.log(2 * math.pi) * log_std.numel() - log_std.sum()
+    std = img[off[N.POLICY_LAYOUT_STD]: off[N.POLICY_LAYOUT_LOGNORM]]
+    std.zero_()
+    std[:d_act].copy_(log_std.exp())
+    img[off[N.POLICY_LAYOUT_LOGNORM]:].zero_()
+    img[off[N.POLICY_LAYOUT_LOGNORM]] = -0.5 * math.log(2 * math.pi) * log_std.numel() - log_std.sum()
     return img
 
 
@@ -132,11 +144,12 @@ class RolloutCollector:
 
     `actions` holds the UN-clipped Gaussian samples and `logp` their log-density (what PPO2's runner stores);
     the env is stepped with `clip(actions, -1, 1)`.  `fused="fp32"` runs policy + env for all T steps
-    in one kernel launch (`roboy_policy_rollout`, float32 FFMA2 -- agrees with the torch policy to ~1e-6);
+    in one kernel launch (`roboy_policy_rollout`, float32 FFMA2 -- agrees with the torch policy to ~1e-6), on every robot;
     `fused="tc"` does the same with the matrix products on the tensor cores (`roboy_policy_rollout_tc`,
     tcgen05 with float16 operands and float32 accumulation -- agrees to ~1e-3, several times faster);
     `fused="tc_exact"` splits every operand into two float16 halves (three MMAs per product) and keeps the accurate
-    tanh -- agrees to ~1e-6 like "fp32", at more than twice its speed; `fused=True` selects it.  (`logp` is always the density of the stored
+    tanh -- agrees to ~1e-6 like "fp32", at more than twice its speed; `fused=True` selects it.  The tensor-core variants
+    run on MSJ-shaped robots only.  (`logp` is always the density of the stored
     sample under the mean the kernel computed; with "tc" that mean differs from the float32 policy's by ~1e-3, so a
     PPO ratio evaluated in float32 starts within ~1e-3 * |z| / std of 1 -- use "tc_exact" or "fp32" where that matters.)  Fused, the Gaussian noise comes from Philox keyed by
     `noise_seed` instead of torch's generator."""
@@ -154,8 +167,9 @@ class RolloutCollector:
         dev, T, N = self.client.device, self.T, self.N
         f32 = dict(dtype=torch.float32, device=dev)
         d_obs, d_act = self.client.dim_obs, self.client.dim_action
-        if self.fused and not self.client.msj_kernels:
-            raise ValueError("the fused policy rollouts are built for MSJ-shaped robots; use fused=False for this robot")
+        if self.fused in ("tc", "tc_exact") and not self.client.msj_kernels:
+            raise ValueError('the tensor-core policy rollouts (fused=True, "tc", "tc_exact") are built for MSJ-shaped robots; '
+                             'use fused="fp32" for this robot')
         self.obs = torch.zeros((T + 1, N, d_obs), **f32)
         self.actions = torch.zeros((T, N, d_act), **f32)
         self.logp = torch.zeros((T, N), **f32)
@@ -168,10 +182,10 @@ class RolloutCollector:
         self._clipped = torch.zeros((N, d_act), **f32)
         self._image, self._image_key = None, None
         if self.fused == "fp32":
-            self._image = torch.zeros(_native.POLICY_IMAGE_FLOATS, **f32)
+            self._image = torch.zeros(_native.policy_layout(d_obs, d_act)[_native.POLICY_LAYOUT_FLOATS], **f32)
         elif self.fused in ("tc", "tc_exact"):
             self._image = torch.zeros(_native.TC_IMAGE_BYTES, dtype=torch.uint8, device=dev)
-        self.noise = None   # tests: set to a [T, N, 8] float32 tensor to have the fused kernel record its noise
+        self.noise = None   # tests: set to a [T, N, A] float32 tensor to have the fused kernel record its noise
         self.obs[0].copy_(env.reset())
 
     def _fused_loop(self):

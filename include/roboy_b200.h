@@ -334,23 +334,24 @@ int roboy_gae(uint64_t T, uint64_t n, const float *reward_dev, const float *valu
 /* Closed-loop rollout with the policy INSIDE the kernel (SURVEY.md 8f row 1; BASELINE.json configs[4]):
  * T steps of [MlpPolicy forward -> Gaussian sample -> clip to the action space -> RoboyEnv.step] for every
  * env in ONE launch -- the loop stable-baselines' PPO2 runner drives over a SubprocVecEnv in
- * train_parallel.py:28-35.  The policy is stable-baselines' MlpPolicy shape: separate 9-64-64 tanh
- * networks for the action mean (8 outputs) and the value (1 output), state-independent log-std.
- * Each env's observation, goal and step counter stay in registers for the T steps; per env-step the
- * kernel writes action 32 + logp 4 + value 4 + obs 36 + reward 4 + done 1 = 81 bytes and reads nothing.
+ * train_parallel.py:28-35.  The policy is stable-baselines' MlpPolicy shape: separate D-64-64 tanh networks
+ * (D = 3J inputs) for the action mean (A outputs) and the value (1 output), state-independent log-std.
+ * Runs on every robot: MSJ-shaped handles (3 joints, 8 tendons, uniform bounds) on the tuned MSJ kernel, every
+ * other robot (and MSJ under ROBOY_B200_FORCE_GENERIC=1) on the generic one.  Each env's observation, goal and
+ * step counter stay on chip for the T steps; per env-step the kernel writes action 4A + logp 4 + value 4 +
+ * obs 12J + reward 4 + done 1 = 4A + 12J + 13 bytes (81 for MSJ) and reads nothing.
  * Env outputs are bit-identical to T roboy_step calls on clip(actions, -1, 1).
  *
- * image_dev: the policy packed as float32 [ROBOY_POLICY_IMAGE_FLOATS], 16-byte aligned.  One network
- * is  W1^T [9][64] | b1 [64] | W2^T [64][64] | b2 [64] | W3^T [64][8] | b3 [8]  (the value network's
- * output layer zero-padded from 1 to 8 columns); the image is  value net | policy net | std [8]
- * (= exp(log_std)) | lognorm (= -0.5*8*log(2 pi) - sum(log_std)) | 3 floats of padding.
- * Noise: Philox4x32-10 keyed by noise_seed, counter (global env id, env call counter, stream 4),
- * Box-Muller; independent of how envs are sharded.
- *   obs_dev     float32 [T+1][n][9]  slot 0 = the observation to start from (input), slots 1..T written
- *   actions_dev float32 [T][n][8]    the UN-clipped samples (what PPO2's runner stores; env.step saw the clip)
+ * image_dev: the policy packed as float32 [offsets[ROBOY_POLICY_LAYOUT_FLOATS]] of roboy_policy_layout(3J, A),
+ * 16-byte aligned (for MSJ that is [ROBOY_POLICY_IMAGE_FLOATS] at the ROBOY_POLICY_OFF_* offsets below).
+ * Noise: Philox4x32-10 keyed by noise_seed, counter (global env id, env call counter, stream 4, sub = k / 4),
+ * Box-Muller on word pair (k % 4) / 2 of that block, its first or second value by k % 2, for normal k = 0..A-1;
+ * independent of how envs are sharded.
+ *   obs_dev     float32 [T+1][n][3J] slot 0 = the observation to start from (input), slots 1..T written
+ *   actions_dev float32 [T][n][A]    the UN-clipped samples (what PPO2's runner stores; env.step saw the clip)
  *   logp_dev    float32 [T][n]       log-density of the sample;  values_dev float32 [T+1][n] (slot T: bootstrap)
- *   reward_dev  float32 [T][n];  done_dev uint8 [T][n];  noise_dev float32 [T][n][8] or NULL (tests)
- * envs_per_thread: 0 = automatic (1 while all envs fit on the chip at once, else 2). */
+ *   reward_dev  float32 [T][n];  done_dev uint8 [T][n];  noise_dev float32 [T][n][A] or NULL (tests)
+ * envs_per_thread: 0 = automatic (MSJ: 1 while all envs fit on the chip at once, else 2; other robots: 1). */
 #define ROBOY_POLICY_HIDDEN 64
 #define ROBOY_POLICY_OFF_W1 0
 #define ROBOY_POLICY_OFF_B1 576
@@ -364,11 +365,38 @@ int roboy_gae(uint64_t T, uint64_t n, const float *reward_dev, const float *valu
 #define ROBOY_POLICY_OFF_STD 10640
 #define ROBOY_POLICY_OFF_LOGNORM 10648
 #define ROBOY_POLICY_IMAGE_FLOATS 10652
+/* Layout of the policy image of roboy_policy_rollout for dim_obs = D = 3J (J = 1..15) and dim_action = A (1..64),
+ * in floats; a pure function (no GPU needed).  One network with W output columns is
+ *   W1^T [D][64] | b1 [64] | W2^T [64][64] | b2 [64] | W3^T [64][W] | b3 [W]
+ * i.e. W1 at 0, b1 at 64D, W2 at 64D + 64, b2 at 64D + 4160, W3 at 64D + 4224, b3 at 64D + 4224 + 64W, and
+ * 64D + 4224 + 65W floats in all.  The image is
+ *   value net (W = 8: the output column zero-padded from 1 to 8) | policy net (W = A8 = 8 * ceil(A / 8), zero-padded
+ *   from A) | std [A8] (= exp(log_std), zero-padded) | lognorm (= -0.5*A*log(2 pi) - sum(log_std)) | padding to a
+ *   multiple of 4 floats,
+ * so every section starts 16-byte aligned.  For D = 9, A = 8 this is the ROBOY_POLICY_OFF_* image above.
+ * offsets[ROBOY_POLICY_LAYOUT_WORDS] receives: W1, B1, W2, B2, W3 (within either network), the b3 of the value net
+ * and of the policy net (within its network), the start of the value net, the policy net, std, lognorm, and the total.
+ * Returns ROBOY_E_ARG for dims outside those ranges. */
+#define ROBOY_POLICY_LAYOUT_W1 0
+#define ROBOY_POLICY_LAYOUT_B1 1
+#define ROBOY_POLICY_LAYOUT_W2 2
+#define ROBOY_POLICY_LAYOUT_B2 3
+#define ROBOY_POLICY_LAYOUT_W3 4
+#define ROBOY_POLICY_LAYOUT_VF_B3 5
+#define ROBOY_POLICY_LAYOUT_PI_B3 6
+#define ROBOY_POLICY_LAYOUT_VF 7
+#define ROBOY_POLICY_LAYOUT_PI 8
+#define ROBOY_POLICY_LAYOUT_STD 9
+#define ROBOY_POLICY_LAYOUT_LOGNORM 10
+#define ROBOY_POLICY_LAYOUT_FLOATS 11
+#define ROBOY_POLICY_LAYOUT_WORDS 12
+int roboy_policy_layout(int dim_obs, int dim_action, uint32_t *offsets);
 int roboy_policy_rollout(roboy_env *env, uint32_t T, const float *image_dev, uint64_t noise_seed, float *obs_dev,
                          float *actions_dev, float *logp_dev, float *values_dev, float *reward_dev, uint8_t *done_dev,
                          float *noise_dev, int envs_per_thread, void *stream);
 /* The same rollout with the two networks' matrix products on the tensor cores (tcgen05.mma kind::f16, M = 128
- * envs per tile, float32 accumulators in tensor memory).  Env outputs remain bit-identical to T roboy_step calls on
+ * envs per tile, float32 accumulators in tensor memory); MSJ-shaped handles only (ROBOY_E_ARG otherwise: other
+ * robots run roboy_policy_rollout).  Env outputs remain bit-identical to T roboy_step calls on
  * clip(actions, -1, 1).  Two precisions:
  *   exact = 0  float16 operands (10-bit mantissa, as TF32), float32 accumulation, tanh.approx: action means and values
  *              agree with the float32 policy to ~1e-3.  The fastest path.
@@ -404,7 +432,8 @@ int roboy_policy_rollout(roboy_env *env, uint32_t T, const float *image_dev, uin
 int roboy_policy_rollout_tc(roboy_env *env, uint32_t T, const float *tc_image_dev, uint64_t noise_seed, float *obs_dev,
                             float *actions_dev, float *logp_dev, float *values_dev, float *reward_dev, uint8_t *done_dev,
                             float *noise_dev, int tiles_per_group, int exact, void *stream);
-/* Launch geometry roboy_policy_rollout uses for this handle (bench.py / tests). */
+/* Launch geometry roboy_policy_rollout uses for this handle (bench.py / tests); ept = envs per thread.  Refuses the
+ * envs_per_thread values roboy_policy_rollout refuses (robots other than MSJ: 0 or 1). */
 int roboy_policy_geometry(roboy_env *env, int envs_per_thread, int *grid, int *block, int *smem_bytes, int *ept);
 int roboy_policy_tc_geometry(roboy_env *env, int tiles_per_group, int exact, int *grid, int *block, int *smem_bytes, int *tpg);
 
