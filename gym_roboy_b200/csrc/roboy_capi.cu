@@ -236,13 +236,9 @@ struct roboy_env {
     uint32_t goal_sub = 0;  // goal draws already made at this call counter (un-fused API)
     uint64_t launches = 0;  // kernels launched through this handle
     PhiloxKeys keys;
-    RobotSpec spec;         // the robot, per component (generic kernels; all robots)
+    RobotSpec spec;         // the robot, per component: the one description of it (tune_step_params reads component 0)
     int J = ROBOY_DIM_JOINT, A = ROBOY_DIM_ACTION, D = ROBOY_DIM_OBS;
     bool msj_shaped = true;  // MSJ's dims with uniform bounds: the tuned step / rollout kernels apply
-    RobotConsts consts;     // ... and their scalar constants
-    FastConsts fast;
-    float act_slope = 0.f, act_hi = 0.f;
-    float hold_lo = 1.f, hold_hi = -1.f;
     int fastdiv = kDivIeee;      // division mode of the tuned MSJ-shaped kernels (msj_math.cuh): IEEE / proved offline / proved at create
     // HBM
     float *goal = nullptr;
@@ -333,8 +329,6 @@ void set_penalty_f32(roboy_env *e) {
         pen.hi_in = round_down_f32(hi - band_hi);
     }
     e->spec.pen = pen;
-    e->fast.pen = pen;
-    e->fast.v_gz_f = (float)e->fast.v_gz;
     for (int k = 0; k < r.J; ++k) e->spec.v_gz_f[k] = (float)r.v_gz[k];
 }
 
@@ -348,35 +342,21 @@ CallCounter counter(roboy_env *e, CallCounter::Mode mode, unsigned long long t_f
     return c;
 }
 
-void fill_step_params(roboy_env *e, StepParams &p, const float *actions, float *obs, float *reward, uint8_t *done) {
+// The fields both step parameter blocks carry (StepParams of the tuned kernels, GStepParams of the generic ones).
+template <class P>
+void fill_common_step_params(roboy_env *e, P &p, const float *actions, float *obs, float *reward, uint8_t *done) {
     p.n = e->cfg.n_envs;
     p.e_begin = 0;
     p.e_end = e->cfg.n_envs;
     p.gid_base = e->cfg.env_id_base;
     p.cc = counter(e, CallCounter::kAdvance);
     p.keys = e->keys;
-    p.c = e->consts;
-    p.f = e->fast;
-    p.f.reward_lo_f = round_up_f32(e->consts.reward_lo);
-    p.f.reward_hi_f = round_down_f32(e->consts.reward_hi);
-    p.hold_lo = e->hold_lo;
-    p.hold_hi = e->hold_hi;
-    p.hold_mag = fmaxf(fabsf(e->hold_lo), fabsf(e->hold_hi));
-    p.hold_c = e->spec.hold_c;
-    p.hold_h = e->spec.hold_h;
-    p.act_in_hi = 1.0f;   // roboy_env.py:31
-    p.act_in_lo = -1.0f;
-    p.act_hi = e->act_hi;
-    p.act_slope = e->act_slope;
     p.max_len = e->cfg.max_episode_len;
     p.actions = actions;
     p.goal = e->goal;
-    p.goal1 = e->goal + e->cfg.n_envs;
-    p.goal2 = e->goal + 2 * e->cfg.n_envs;
     p.step_flags = e->step_flags;
     p.held = e->held;
     p.obs = obs ? obs : e->obs;
-    p.obs_aligned = ((uintptr_t)p.obs & 15) == 0;
     p.reward = reward ? reward : e->reward;
     p.done = done ? done : e->done;
     p.terminal_obs = e->terminal_obs;
@@ -386,30 +366,62 @@ void fill_step_params(roboy_env *e, StepParams &p, const float *actions, float *
     p.first_bad = e->first_bad;
 }
 
+// The scalar constants of the tuned MSJ-shaped kernels: component 0 of the finished RobotSpec (an MSJ-shaped robot has
+// the same bounds on every component), after prove_generic_fastdiv and set_penalty_f32.  Kept in the parameter block as
+// scalars: the tuned step is launch-bound at small sizes, and carrying the whole RobotSpec there made it slower.
+void tune_step_params(const RobotSpec &r, int div_mode, StepParams &p) {
+    RobotConsts &c = p.c;
+    c.a_hi = r.a_hi[0];
+    c.a_lo = r.a_lo[0];
+    c.a_span = r.a_span[0];
+    c.v_hi = r.v_hi[0];
+    c.v_lo = r.v_lo[0];
+    c.v_span = r.v_span[0];
+    c.thr_angle = r.thr_angle;
+    c.thr_vel = r.thr_vel;
+    c.penalty_boundary = r.penalty_boundary;
+    c.bonus_goal = r.bonus_goal;
+    c.reward_lo = r.reward_lo;
+    c.reward_hi = r.reward_hi;
+    FastConsts &f = p.f;
+    if (div_mode == kDivChecked) {   // the reciprocals prove_generic_fastdiv checked on this device
+        f.a_rc = r.a_rcp[0];
+        f.v_rc = r.v_rcp[0];
+    } else {                         // kDivProved: the reciprocals oracle/verify_fastdiv.c proved (unused under kDivIeee)
+        f.a_rc = (float)(1.0 / (double)r.a_span[0]);
+        f.v_rc = (float)(1.0 / (double)r.v_span[0]);
+    }
+    f.thr_angle_sq_hi = r.thr_angle_sq_hi;
+    f.a_span24 = r.a_span[0] * 0x1p-24f;
+    f.a_span21 = r.a_span21[0];
+    f.reward_lo_f = round_up_f32(r.reward_lo);
+    f.reward_hi_f = round_down_f32(r.reward_hi);
+    f.v_gz = r.v_gz[0];
+    f.v_gz_f = r.v_gz_f[0];
+    f.pen = r.pen;
+    p.hold_lo = r.hold_lo[0];
+    p.hold_hi = r.hold_hi[0];
+    p.hold_mag = fmaxf(fabsf(r.hold_lo[0]), fabsf(r.hold_hi[0]));
+    p.hold_c = r.hold_c;
+    p.hold_h = r.hold_h;
+    p.act_in_hi = 1.0f;   // roboy_env.py:31
+    p.act_in_lo = -1.0f;
+}
+
+void fill_step_params(roboy_env *e, StepParams &p, const float *actions, float *obs, float *reward, uint8_t *done) {
+    fill_common_step_params(e, p, actions, obs, reward, done);
+    tune_step_params(e->spec, e->fastdiv, p);
+    p.goal1 = e->goal + e->cfg.n_envs;
+    p.goal2 = e->goal + 2 * e->cfg.n_envs;
+    p.obs_aligned = ((uintptr_t)p.obs & 15) == 0;
+}
+
 void fill_generic_step_params(roboy_env *e, GStepParams &p, const float *actions, float *obs, float *reward, uint8_t *done) {
-    p.n = e->cfg.n_envs;
-    p.e_begin = 0;
-    p.e_end = e->cfg.n_envs;
-    p.gid_base = e->cfg.env_id_base;
-    p.cc = counter(e, CallCounter::kAdvance);
-    p.keys = e->keys;
+    fill_common_step_params(e, p, actions, obs, reward, done);
     p.r = e->spec;
-    p.max_len = e->cfg.max_episode_len;
     p.penalty = e->cfg.joint_vel_penalty;
     p.bonus = e->cfg.bonus_for_goal;
     p.auto_reset = e->cfg.auto_reset;
-    p.actions = actions;
-    p.goal = e->goal;
-    p.step_flags = e->step_flags;
-    p.held = e->held;
-    p.obs = obs ? obs : e->obs;
-    p.reward = reward ? reward : e->reward;
-    p.done = done ? done : e->done;
-    p.terminal_obs = e->terminal_obs;
-    p.done_bits = e->done_bits;
-    p.stats = e->stats;
-    p.err_flags = e->err_flags;
-    p.first_bad = e->first_bad;
 }
 
 // One fused step over local envs [e_begin, e_end): the tuned kernel for MSJ-shaped robots, the generic one otherwise.
@@ -525,40 +537,7 @@ int roboy_create(const roboy_cfg *cfg, int device, roboy_env **out) {
     e->msj_shaped = is_msj_shaped(*cfg, r);
     if (const char *force = getenv("ROBOY_B200_FORCE_GENERIC"))   // tests: run an MSJ-shaped robot through the generic kernels
         if (force[0] == '1') e->msj_shaped = false;
-    // scalar constants of the tuned MSJ-shaped kernels (component 0 stands for all when msj_shaped)
-    RobotConsts &c = e->consts;
-    c.a_hi = r.a_hi[0];
-    c.a_lo = r.a_lo[0];
-    c.a_span = r.a_hi[0] - r.a_lo[0];
-    c.v_hi = r.v_hi[0];
-    c.v_lo = r.v_lo[0];
-    c.v_span = r.v_hi[0] - r.v_lo[0];
-    c.thr_angle = r.thr_angle;
-    c.thr_vel = r.thr_vel;
-    c.penalty_boundary = r.penalty_boundary;
-    c.bonus_goal = r.bonus_goal;
-    c.reward_lo = cfg->reward_lo;
-    c.reward_hi = cfg->reward_hi;
-    const float act_lo0 = cfg->per_component_bounds ? cfg->act_low_v[0] : cfg->act_low;
-    const float act_hi0 = cfg->per_component_bounds ? cfg->act_high_v[0] : cfg->act_high;
-    e->act_hi = act_hi0;
-    e->act_slope = (act_hi0 - act_lo0) / (1.0f - (-1.0f));  // roboy_env.py:157, float32
-    e->hold_lo = r.hold_lo[0];
-    e->hold_hi = r.hold_hi[0];
-    e->fast.a_rc = (float)(1.0 / (double)c.a_span);
-    e->fast.v_rc = (float)(1.0 / (double)c.v_span);
-    e->fast.thr_angle_sq_hi = round_up_f32((double)c.thr_angle * (double)c.thr_angle * (1.0 + 1e-5));
-    e->fast.a_span24 = c.a_span * 0x1p-24f;
-    e->fast.a_span21 = c.a_span * 0x1p-21f;
-    e->fast.reward_lo_f = -INFINITY;
-    e->fast.reward_hi_f = INFINITY;
-    {   // roboy_robot.py:93-95 on the float64 zero velocity of the goal (roboy_env.py:23): (2*0 - max - min) / (max - min)
-        volatile double t = 2.0 * 0.0;
-        t = t - (double)c.v_hi;
-        t = t - (double)c.v_lo;
-        e->fast.v_gz = t / (double)c.v_span;
-    }
-    e->fastdiv = (e->msj_shaped && spans_are_proved(c.a_lo, c.a_hi, c.v_lo, c.v_hi)) ? kDivProved : kDivIeee;
+    e->fastdiv = (e->msj_shaped && spans_are_proved(r.a_lo[0], r.a_hi[0], r.v_lo[0], r.v_hi[0])) ? kDivProved : kDivIeee;
     if (e->fastdiv == kDivIeee) {
         // Any other robot: the division by its spans is checked against IEEE division on this device, over all 2^32
         // numerators (roboy_generic.cuh).  The generic step uses the per-joint reciprocals; an MSJ-shaped robot with other
@@ -570,11 +549,7 @@ int roboy_create(const roboy_cfg *cfg, int device, roboy_env **out) {
                 free_env(e);
                 return fail(ROBOY_E_CUDA, "fast-division proof: %s", cudaGetErrorString(perr));
             }
-            if (e->msj_shaped && e->spec.fastdiv) {
-                e->fastdiv = kDivChecked;
-                e->fast.a_rc = e->spec.a_rcp[0];
-                e->fast.v_rc = e->spec.v_rcp[0];
-            }
+            if (e->msj_shaped && e->spec.fastdiv) e->fastdiv = kDivChecked;
         }
     }
 
@@ -645,8 +620,8 @@ int roboy_destroy(roboy_env *env) {
 
 int roboy_set_reward_range(roboy_env *env, double lo, double hi) {
     if (check_env(env)) return ROBOY_E_ARG;
-    env->cfg.reward_lo = env->consts.reward_lo = env->spec.reward_lo = lo;
-    env->cfg.reward_hi = env->consts.reward_hi = env->spec.reward_hi = hi;
+    env->cfg.reward_lo = env->spec.reward_lo = lo;
+    env->cfg.reward_hi = env->spec.reward_hi = hi;
     set_penalty_f32(env);
     return ROBOY_OK;
 }

@@ -62,7 +62,8 @@ struct StepParams {
                                  // |fl(fl(slope*fl(a - in_hi)) + act_hi)| <= 1e-8, i.e. numpy's
                                  // allclose(rescaled, 0) (roboy_env.py:157-158, simulation_client.py:38)
     float act_in_hi, act_in_lo;  // RoboyEnv.action_space bounds, roboy_env.py:31
-    float act_hi, act_slope;     // robot action space high and fl32((hi-lo)/(in_hi-in_lo)), roboy_env.py:157
+    float pad_[2];               // unread; without it the pointers below sit 8 bytes earlier and ptxas pairs their constant
+                                 // loads differently in the step and open-loop kernels
     int32_t max_len;             // roboy_env.py:28
     int32_t obs_aligned;         // obs pointer is 16-byte aligned: vector / bulk stores allowed
     // inputs / state / outputs (device pointers)
