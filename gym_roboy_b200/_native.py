@@ -110,6 +110,7 @@ SIGNATURES = {
     "roboy_gae": (_int, [_u64, _u64, _vp, _vp, _vp, _vp, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp]),
     "roboy_policy_rollout": (_int, [_vp, ctypes.c_uint32, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _vp]),
     "roboy_policy_rollout_tc": (_int, [_vp, ctypes.c_uint32, _vp, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _vp]),
+    "roboy_policy_evaluate": (_int, [_vp, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32, _vp, _vp, _vp, _vp, _vp]),
     "roboy_policy_tc_geometry": (_int, [_vp, _int, _int, ctypes.POINTER(_int), ctypes.POINTER(_int), ctypes.POINTER(_int),
                                         ctypes.POINTER(_int)]),
     "roboy_policy_layout": (_int, [_int, _int, ctypes.POINTER(ctypes.c_uint32)]),

@@ -1415,6 +1415,40 @@ int roboy_policy_rollout_tc(roboy_env *env, uint32_t T, const float *tc_image_de
                                  done_dev, noise_dev, tiles_per_group, stream);
 }
 
+int roboy_policy_evaluate(roboy_env *env, uint32_t T, const float *image_dev, float *obs_dev, uint32_t episodes,
+                          double *returns_dev, uint32_t *lengths_dev, uint8_t *reached_dev, uint32_t *completed_dev,
+                          void *stream) {
+    if (check_env(env)) return ROBOY_E_ARG;
+    if (!env->cfg.auto_reset)
+        return fail(ROBOY_E_ARG, "roboy_policy_evaluate needs auto_reset: without it no new episode ever starts");
+    if (!image_dev || !obs_dev || !returns_dev || !lengths_dev || !reached_dev || !completed_dev)
+        return fail(ROBOY_E_ARG, "NULL device pointer");
+    if ((uintptr_t)image_dev & 15) return fail(ROBOY_E_ARG, "image must be 16-byte aligned");
+    if ((uintptr_t)obs_dev & 3) return fail(ROBOY_E_ARG, "obs must be 4-byte aligned");
+    if (T == 0) return ROBOY_OK;
+    DeviceGuard g(env->device);
+    env->goal_sub = 1;
+    // every robot, MSJ-shaped ones included, on the generic env step
+    GStepParams p;
+    fill_generic_step_params(env, p, nullptr, nullptr, nullptr, nullptr);
+    p.cc.advance = T;
+    p.done_bits = nullptr;   // the done-index list belongs to single steps
+    GEvalParams q{};
+    q.image = image_dev;
+    if (roboy_policy_layout(env->D, env->A, q.off) != ROBOY_OK) return ROBOY_E_ARG;
+    q.T = T;
+    q.episodes = episodes;
+    q.obs_aligned = ((uintptr_t)obs_dev & 15) == 0;   // one [n][3J] block: every chunk of 32 rows starts 16-byte aligned
+    q.obs = obs_dev;
+    q.returns = returns_dev;
+    q.lengths = lengths_dev;
+    q.reached = reached_dev;
+    q.completed = completed_dev;
+    CUDA_TRY(launch_generic_policy_evaluate(p, q, env->sm_count, (cudaStream_t)stream));
+    env->launches++;
+    return ROBOY_OK;
+}
+
 int roboy_policy_tc_geometry(roboy_env *env, int tiles_per_group, int exact, int *grid, int *block, int *smem_bytes, int *tpg) {
     if (check_env(env)) return ROBOY_E_ARG;
     const PolicyGeom geo = policy_tc_geometry(env->cfg.n_envs, env->sm_count, tiles_per_group, exact != 0);

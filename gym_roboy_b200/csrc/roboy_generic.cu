@@ -231,7 +231,7 @@ __global__ void __launch_bounds__(g_step_block(JM), g_min_blocks(JM)) generic_st
         }
 
         const bool done = generic_env_step<JM>(p, FASTDIV, live, hold, act_ok, q, qd, g, sf, gid, t, e, n_envs, s_cnt, &s_eplen,
-                                               sum_reward, [&](uint32_t word, float rf, bool d) {
+                                               sum_reward, [&](uint32_t word, float rf, bool d, bool) {
                                                    p.step_flags[e] = word;
                                                    p.reward[e] = rf;
                                                    p.done[e] = (uint8_t)d;

@@ -68,4 +68,21 @@ struct GPolicyParams {
 PolicyGeom generic_policy_geometry(int J, uint32_t image_floats, uint64_t n_envs, int sm_count);
 cudaError_t launch_generic_policy_rollout(const GStepParams &p, const GPolicyParams &q, int sm_count, cudaStream_t stream);
 
+// Deterministic policy evaluation for every robot (roboy_policy_eval.cu): the rollout's loop with the action
+// clip(mean(obs), -1, 1), no value network and no per-step stores; each env's episodes are recorded as they finish.
+// p is as for launch_generic_step (p.actions, p.obs, p.reward and p.done are not used).
+struct GEvalParams {
+    const float *__restrict__ image;  // the roboy_policy_layout(3J, A) image; only its policy net is read
+    uint32_t off[ROBOY_POLICY_LAYOUT_WORDS];
+    uint32_t T;
+    uint32_t episodes;                // records per env (K)
+    int32_t obs_aligned;              // obs is 16-byte aligned
+    float *__restrict__ obs;          // [n][3J] in: the observation to start from; out: the one after the last step
+    double *__restrict__ returns;     // [K][n]
+    uint32_t *__restrict__ lengths;   // [K][n]
+    uint8_t *__restrict__ reached;    // [K][n]
+    uint32_t *__restrict__ completed; // [n]
+};
+cudaError_t launch_generic_policy_evaluate(const GStepParams &p, const GEvalParams &q, int sm_count, cudaStream_t stream);
+
 }  // namespace roboy

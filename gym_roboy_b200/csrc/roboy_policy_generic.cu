@@ -24,6 +24,7 @@
 #include "../../include/roboy_b200.h"
 #include "generic_env.cuh"
 #include "policy_common.cuh"
+#include "policy_generic.cuh"
 #include "roboy_generic.cuh"
 #include "roboy_policy.cuh"
 
@@ -31,55 +32,7 @@ namespace roboy {
 
 namespace {
 
-constexpr int kGHid = ROBOY_POLICY_HIDDEN;  // 64
 constexpr int kGPolicySmemBudget = 227 * 1024;
-
-// tanh(h2) of one network into the thread's hidden column hs[j * 32] (j = 0..63); `row` is the env's observation row
-template <int D>
-__device__ __forceinline__ void mlp_hidden(const float *__restrict__ net, const uint32_t (&off)[ROBOY_POLICY_LAYOUT_WORDS],
-                                           const float *__restrict__ row, float *__restrict__ hs) {
-    float2 acc[1][32];
-    load_bias64<1>(net + off[ROBOY_POLICY_LAYOUT_B1], acc);
-    dense64<1>(net + off[ROBOY_POLICY_LAYOUT_W1], row, D, 1, 0, acc);
-#pragma unroll
-    for (int j2 = 0; j2 < 32; ++j2) {
-        hs[(2 * j2) * 32] = tanh_mufu(acc[0][j2].x);
-        hs[(2 * j2 + 1) * 32] = tanh_mufu(acc[0][j2].y);
-    }
-    load_bias64<1>(net + off[ROBOY_POLICY_LAYOUT_B2], acc);
-    dense64<1>(net + off[ROBOY_POLICY_LAYOUT_W2], hs, kGHid, 32, 0, acc);
-#pragma unroll
-    for (int j2 = 0; j2 < 32; ++j2) {
-        hs[(2 * j2) * 32] = tanh_mufu(acc[0][j2].x);
-        hs[(2 * j2 + 1) * 32] = tanh_mufu(acc[0][j2].y);
-    }
-}
-
-// Output columns 8c .. 8c + 7 of the last layer: b3 + sum_j tanh(h2_j) * W3[j] (W3 is [64][W], b3 [W])
-__device__ __forceinline__ void mlp_out8(const float *__restrict__ w3, const float *__restrict__ b3, int W, int c,
-                                         const float *__restrict__ hs, float (&out)[8]) {
-    const float4 b0 = reinterpret_cast<const float4 *>(b3 + 8 * c)[0];
-    const float4 b1 = reinterpret_cast<const float4 *>(b3 + 8 * c)[1];
-    float2 o[4] = {make_float2(b0.x, b0.y), make_float2(b0.z, b0.w), make_float2(b1.x, b1.y), make_float2(b1.z, b1.w)};
-    const float *w = w3 + 8 * c;
-#pragma unroll 8
-    for (int j = 0; j < kGHid; ++j) {
-        const float4 wa = reinterpret_cast<const float4 *>(w + j * W)[0], wb = reinterpret_cast<const float4 *>(w + j * W)[1];
-        const float t = hs[j * 32];
-        const float2 tt = make_float2(t, t);
-        o[0] = __ffma2_rn(make_float2(wa.x, wa.y), tt, o[0]);
-        o[1] = __ffma2_rn(make_float2(wa.z, wa.w), tt, o[1]);
-        o[2] = __ffma2_rn(make_float2(wb.x, wb.y), tt, o[2]);
-        o[3] = __ffma2_rn(make_float2(wb.z, wb.w), tt, o[3]);
-    }
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        out[2 * k] = o[k].x;
-        out[2 * k + 1] = o[k].y;
-    }
-}
-
-__host__ __device__ constexpr int g_stage_stride(int J) { return (3 * J) | 1; }
 
 }  // namespace
 
@@ -205,7 +158,7 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_rollout_ke
                 for (int k = 0; k < JM; ++k) qds[k] = g_draw_value(r, p.keys, gid, t, cur, J + k, k);
             }
             const bool done = generic_env_step<JM>(p, fastdiv, live, hold, act_ok, qs, qds, g, sf, gid, t, env, n_envs, s_cnt,
-                                                   eplen_counter(s_cnt), sum_reward, [&](uint32_t word, float rf, bool d) {
+                                                   eplen_counter(s_cnt), sum_reward, [&](uint32_t word, float rf, bool d, bool) {
                                                        sf = word;
                                                        p.reward[slot] = rf;
                                                        p.done[slot] = (uint8_t)d;

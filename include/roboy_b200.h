@@ -432,6 +432,36 @@ int roboy_policy_rollout(roboy_env *env, uint32_t T, const float *image_dev, uin
 int roboy_policy_rollout_tc(roboy_env *env, uint32_t T, const float *tc_image_dev, uint64_t noise_seed, float *obs_dev,
                             float *actions_dev, float *logp_dev, float *values_dev, float *reward_dev, uint8_t *done_dev,
                             float *noise_dev, int tiles_per_group, int exact, void *stream);
+/* Deterministic evaluation of a policy (stable-baselines' evaluate_policy(model, env, n_eval_episodes,
+ * deterministic=True)) in ONE launch, on every robot: each env plays T steps of the policy mean and records its episodes
+ * as they finish; nothing grows with T.  The contract:
+ *  1. Image: image_dev is the roboy_policy_layout(3J, A) image of roboy_policy_rollout.  Only the policy net is read;
+ *     the value net, std and lognorm are ignored.
+ *  2. Steps: every env takes exactly T steps, calls t0+1 .. t0+T of the handle's call counter, with the action
+ *     clip(mean(obs), -1, 1); a NaN mean stays NaN (ROBOY_ERR_ACTION, as in the rollouts).  The mean is evaluated with
+ *     the instructions roboy_policy_rollout uses, so the env outputs are those of roboy_policy_rollout with std 0.
+ *  3. State after the call: call counter, goals, step words, error word, first offender and ROBOY_STAT_* advance exactly
+ *     as for T roboy_step calls on those actions.
+ *  4. Observations: obs_dev float32 [n][3J] is read as the observation to start from and overwritten with the
+ *     observation after call T (env.step continues from it).
+ *  5. Which episodes count: an episode counts only if it starts inside the call.  An env whose step counter is at its
+ *     reset value (1) when the call starts begins one at call 1; after every auto-reset inside the call the next
+ *     episode begins at the next call.  An episode already in progress at the call is not counted.
+ *  6. Records: the first `episodes` (K) counted episodes of env e go to slot k * n + e (64-bit) of the [K][n] arrays:
+ *       returns_dev float64  the sum, in step order, of the float32 rewards of the episode (what evaluate_policy sums)
+ *       lengths_dev uint32   step_num - 1 at the done (the term ROBOY_STAT_SUM_EPLEN adds)
+ *       reached_dev uint8    1 if the done came from _did_reach_goal (also on a step that times out as well)
+ *     Slots not filled hold NaN, 0, 0.  completed_dev uint32 [n]: every counted episode of env e that finished,
+ *     including those beyond K.
+ *  7. Refusals (ROBOY_E_ARG with a message): auto_reset off (no new episode would ever start), a NULL pointer, an
+ *     image_dev not 16-byte aligned, an obs_dev not 4-byte aligned.  T == 0 returns without a launch (outputs untouched).
+ *  8. Robots: every handle runs the generic env step, MSJ-shaped ones included; their env outputs equal roboy_step's
+ *     bit for bit, except rewards under joint_vel_penalty, which agree to ~2e-7 (relative).
+ *  9. Sharding: results do not depend on it (draws are keyed by global env id).
+ * Per env-step: 64 * (3J + 64 + A8) FMAs (A8 = 8 * ceil(A / 8)); HBM traffic is the records and the goals drawn on done. */
+int roboy_policy_evaluate(roboy_env *env, uint32_t T, const float *image_dev, float *obs_dev, uint32_t episodes,
+                          double *returns_dev, uint32_t *lengths_dev, uint8_t *reached_dev, uint32_t *completed_dev,
+                          void *stream);
 /* Launch geometry roboy_policy_rollout uses for this handle (bench.py / tests); ept = envs per thread.  Refuses the
  * envs_per_thread values roboy_policy_rollout refuses (robots other than MSJ: 0 or 1). */
 int roboy_policy_geometry(roboy_env *env, int envs_per_thread, int *grid, int *block, int *smem_bytes, int *ept);
