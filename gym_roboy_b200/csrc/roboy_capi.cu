@@ -1338,6 +1338,15 @@ int roboy_gae(uint64_t T, uint64_t n, const float *reward_dev, const float *valu
     return ROBOY_OK;
 }
 
+// The env-step block and the image offsets of a T-step fused generic policy launch (the rollout's and the evaluator's)
+static int fill_generic_policy_launch(roboy_env *env, uint32_t T, float *reward_dev, uint8_t *done_dev, GStepParams &p,
+                                      uint32_t (&off)[ROBOY_POLICY_LAYOUT_WORDS]) {
+    fill_generic_step_params(env, p, nullptr, nullptr, reward_dev, done_dev);
+    p.cc.advance = T;
+    p.done_bits = nullptr;   // the done-index list belongs to single steps
+    return roboy_policy_layout(env->D, env->A, off);
+}
+
 static int policy_rollout_common(roboy_env *env, bool tensor_cores, bool exact, uint32_t T, const float *image_dev, uint64_t noise_seed,
                                  float *obs_dev, float *actions_dev, float *logp_dev, float *values_dev, float *reward_dev,
                                  uint8_t *done_dev, float *noise_dev, int envs_per_thread, void *stream) {
@@ -1359,12 +1368,9 @@ static int policy_rollout_common(roboy_env *env, bool tensor_cores, bool exact, 
     env->goal_sub = 1;
     if (!env->msj_shaped) {
         GStepParams p;
-        fill_generic_step_params(env, p, nullptr, nullptr, reward_dev, done_dev);
-        p.cc.advance = T;
-        p.done_bits = nullptr;   // the done-index list belongs to single steps
         GPolicyParams q{};
+        if (fill_generic_policy_launch(env, T, reward_dev, done_dev, p, q.off) != ROBOY_OK) return ROBOY_E_ARG;
         q.image = image_dev;
-        if (roboy_policy_layout(env->D, env->A, q.off) != ROBOY_OK) return ROBOY_E_ARG;
         q.T = T;
         q.obs_aligned = (((uintptr_t)obs_dev & 15) == 0) && (env->cfg.n_envs * env->D * sizeof(float)) % 16 == 0;
         q.obs = obs_dev;
@@ -1430,12 +1436,9 @@ int roboy_policy_evaluate(roboy_env *env, uint32_t T, const float *image_dev, fl
     env->goal_sub = 1;
     // every robot, MSJ-shaped ones included, on the generic env step
     GStepParams p;
-    fill_generic_step_params(env, p, nullptr, nullptr, nullptr, nullptr);
-    p.cc.advance = T;
-    p.done_bits = nullptr;   // the done-index list belongs to single steps
     GEvalParams q{};
+    if (fill_generic_policy_launch(env, T, nullptr, nullptr, p, q.off) != ROBOY_OK) return ROBOY_E_ARG;
     q.image = image_dev;
-    if (roboy_policy_layout(env->D, env->A, q.off) != ROBOY_OK) return ROBOY_E_ARG;
     q.T = T;
     q.episodes = episodes;
     q.obs_aligned = ((uintptr_t)obs_dev & 15) == 0;   // one [n][3J] block: every chunk of 32 rows starts 16-byte aligned

@@ -377,9 +377,7 @@ cudaError_t launch_generic_step(const GStepParams &p, int sm_count, cudaStream_t
             if (p.r.fastdiv) generic_step_kernel<JJ, true><<<grid, block, smem, stream>>>(p); \
             else generic_step_kernel<JJ, false><<<grid, block, smem, stream>>>(p); \
             break;
-        ROBOY_GENERIC_CASE(1) ROBOY_GENERIC_CASE(2) ROBOY_GENERIC_CASE(3) ROBOY_GENERIC_CASE(4) ROBOY_GENERIC_CASE(5)
-        ROBOY_GENERIC_CASE(6) ROBOY_GENERIC_CASE(7) ROBOY_GENERIC_CASE(8) ROBOY_GENERIC_CASE(9) ROBOY_GENERIC_CASE(10)
-        ROBOY_GENERIC_CASE(11) ROBOY_GENERIC_CASE(12) ROBOY_GENERIC_CASE(13) ROBOY_GENERIC_CASE(14) ROBOY_GENERIC_CASE(15)
+        ROBOY_GENERIC_JOINT_COUNTS(ROBOY_GENERIC_CASE)
 #undef ROBOY_GENERIC_CASE
         default: return cudaErrorInvalidValue;
     }

@@ -19,6 +19,8 @@
 namespace roboy {
 
 constexpr int kMaxJoint = 15, kJointPad = 16, kMaxAction = 64;
+// X(J) for every joint count with its own instantiation of the generic kernels: 1..kMaxJoint
+#define ROBOY_GENERIC_JOINT_COUNTS(X) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15)
 
 struct RobotSpec {
     int32_t J, A;                             // joints, tendons; observation rows hold 3 * J floats

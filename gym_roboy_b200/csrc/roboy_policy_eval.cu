@@ -9,7 +9,7 @@
 //     whether that episode counts, how many records it wrote, how many counted episodes finished) and writes a record
 //     [return, length, reached] when a counted episode ends; unfilled records are set to [NaN, 0, 0] at the end;
 //   * the observation after the last step is stored once, coalesced through the warp's stage.
-// The policy mean comes from the rollout's mlp_hidden / mlp_out8 (policy_generic.cuh) and the env step is
+// The frame around the loop body and the policy mean are the rollout's (policy_generic.cuh) and the env step is
 // generic_env_step (generic_env.cuh): the env outputs are those of T roboy_step calls on the clipped means, bit for bit.
 // An episode counts when it starts inside the launch: at the first step for an env whose step counter is 1, and at the
 // step after every done (auto-reset on).  Per env-step the kernel evaluates 64 * (D + 64 + A8) FMAs and writes nothing
@@ -36,17 +36,11 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_evaluate_k
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int n_warps = blockDim.x >> 5;
-    // shared memory: policy net | per warp: hidden column [64][32] | obs stage [32][S] | reduction | counters
-    const uint32_t img_floats = q.off[ROBOY_POLICY_LAYOUT_STD] - q.off[ROBOY_POLICY_LAYOUT_PI];
-    float *pi_net = smem;
-    float *hs = smem + img_floats + warp * (kGHid * 32) + lane;
-    float *stage = smem + img_floats + n_warps * (kGHid * 32) + warp * (32 * S);
-    double *s_red = reinterpret_cast<double *>(smem + img_floats + n_warps * (kGHid * 32 + 32 * S));
-    unsigned int *s_cnt = reinterpret_cast<unsigned int *>(s_red + n_warps);
-    const float4 *src = reinterpret_cast<const float4 *>(q.image + q.off[ROBOY_POLICY_LAYOUT_PI]);
-    for (uint32_t i = threadIdx.x; i < img_floats / 4; i += blockDim.x) reinterpret_cast<float4 *>(pi_net)[i] = src[i];
-    if (threadIdx.x < kCntWords) s_cnt[threadIdx.x] = 0;
-    __syncthreads();
+    // the policy net only; launch_generic_policy_evaluate sizes shared memory from the same difference
+    const uint32_t net_floats = q.off[ROBOY_POLICY_LAYOUT_STD] - q.off[ROBOY_POLICY_LAYOUT_PI];
+    const GPolicySmem m = g_policy_smem<J>(smem, net_floats);
+    g_policy_smem_fill(m, q.image + q.off[ROBOY_POLICY_LAYOUT_PI], net_floats);
+    const float *pi_net = m.image;
 
     const uint64_t t_first = counter_begin(p.cc);
     const uint32_t n_end = (uint32_t)p.e_end, n_envs = (uint32_t)p.n;
@@ -54,7 +48,7 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_evaluate_k
     const uint32_t n_chunks = (n_end + 31) / 32;
     const uint32_t warp_stride = gridDim.x * n_warps;
     const bool fastdiv = r.fastdiv != 0;   // the step kernel's choice (launch_generic_step)
-    float *row = stage + lane * S;
+    float *row = m.stage + lane * S;
     float sum_reward = 0.0f;
 
     for (uint32_t chunk = blockIdx.x * n_warps + warp; chunk < n_chunks; chunk += warp_stride) {
@@ -78,40 +72,24 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_evaluate_k
 
         for (uint32_t tt = 0; tt < q.T; ++tt) {
             // ---- policy network, 8 output columns at a time: mean -> clip -> action tests ----
-            mlp_hidden<D>(pi_net, q.off, row, hs);
+            mlp_hidden<D>(pi_net, q.off, row, m.hs);
             const uint64_t t = t_first + tt;
             bool act_ok = true, hold = live;
             for (int c = 0; c < A8 / 8; ++c) {
                 float mean[8];
-                mlp_out8(pi_net + q.off[ROBOY_POLICY_LAYOUT_W3], pi_net + q.off[ROBOY_POLICY_LAYOUT_PI_B3], A8, c, hs, mean);
+                mlp_out8(pi_net + q.off[ROBOY_POLICY_LAYOUT_W3], pi_net + q.off[ROBOY_POLICY_LAYOUT_PI_B3], A8, c, m.hs, mean);
 #pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    const int k = 8 * c + i;
-                    if (k < A) {
-                        const float cl = fminf(fmaxf(mean[i], -1.0f), 1.0f);
-                        const float a = (mean[i] != mean[i]) ? mean[i] : cl;   // a NaN stays a NaN (and fails the assert)
-                        act_ok = act_ok && (a >= -1.0f && a <= 1.0f);                      // roboy_env.py:52
-                        hold = hold && (a >= r.hold_lo[k] && a <= r.hold_hi[k]);           // simulation_client.py:38
-                    }
-                }
+                for (int i = 0; i < 8; ++i)
+                    if (8 * c + i < A) g_clip_test(r, 8 * c + i, mean[i], act_ok, hold);
             }
 
             // ---- RoboyEnv.step on the clipped mean: the generic step kernel's per-env body ----
             float qs[JM], qds[JM];
-#pragma unroll
-            for (int k = 0; k < JM; ++k) qs[k] = qds[k] = 0.0f;
-            if (live) {
-                DrawCursor cur;
-                cur.block = 0xffffffffu;
-#pragma unroll
-                for (int k = 0; k < JM; ++k) qs[k] = g_draw_value(r, p.keys, gid, t, cur, k, k);
-#pragma unroll
-                for (int k = 0; k < JM; ++k) qds[k] = g_draw_value(r, p.keys, gid, t, cur, J + k, k);
-            }
+            g_draw_step_state<JM>(r, p.keys, live, gid, t, qs, qds);
             const uint32_t step_in = sf & ROBOY_STEP_MASK;
             const uint32_t ep_len = step_in + (step_in < ROBOY_STEP_MASK) - 1u;   // step_num - 1 at a done (:60)
-            generic_env_step<JM>(p, fastdiv, live, hold, act_ok, qs, qds, g, sf, gid, t, env, n_envs, s_cnt,
-                                 eplen_counter(s_cnt), sum_reward, [&](uint32_t word, float rf, bool d, bool reached) {
+            generic_env_step<JM>(p, fastdiv, live, hold, act_ok, qs, qds, g, sf, gid, t, env, n_envs, m.s_cnt,
+                                 eplen_counter(m.s_cnt), sum_reward, [&](uint32_t word, float rf, bool d, bool reached) {
                                      sf = word;
                                      if (counting) {
                                          ret = __dadd_rn(ret, (double)rf);
@@ -132,12 +110,7 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_evaluate_k
                                      }
                                  });
             // ---- the next observation [q, qd, goal] (after a done, g already holds the reset()'s goal) ----
-#pragma unroll
-            for (int k = 0; k < JM; ++k) {
-                row[k] = qs[k];
-                row[J + k] = qds[k];
-                row[2 * J + k] = g[k];
-            }
+            g_stage_obs<JM>(row, qs, qds, g);
         }
         if (live) {
             p.step_flags[env] = sf;
@@ -159,38 +132,30 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_evaluate_k
 #pragma unroll
                 for (int c = 0; c < 4; ++c) {
                     const int i = 4 * i4 + c;
-                    v[c] = stage[(i / D) * S + i % D];
+                    v[c] = m.stage[(i / D) * S + i % D];
                 }
                 dst4[i4] = make_float4(v[0], v[1], v[2], v[3]);
             }
         } else {
             const uint32_t rows = full ? 32u : n_end - base;
-            for (uint32_t i = lane; i < rows * D; i += 32) dst[i] = stage[(i / D) * S + i % D];
+            for (uint32_t i = lane; i < rows * D; i += 32) dst[i] = m.stage[(i / D) * S + i % D];
         }
         __syncwarp();
     }
 
-    policy_stats_tail(p, q.T, t_first, sum_reward, s_red, s_cnt);
+    policy_stats_tail(p, q.T, t_first, sum_reward, m.s_red, m.s_cnt);
 }
 
 cudaError_t launch_generic_policy_evaluate(const GStepParams &p, const GEvalParams &q, int sm_count, cudaStream_t stream) {
     if (p.e_end <= p.e_begin) return cudaSuccess;
-    const uint32_t net_floats = q.off[ROBOY_POLICY_LAYOUT_STD] - q.off[ROBOY_POLICY_LAYOUT_PI];
-    const PolicyGeom g = generic_policy_geometry(p.r.J, net_floats, p.e_end, sm_count);
-    void (*fn)(const GStepParams, const GEvalParams) = nullptr;
     switch (p.r.J) {
 #define ROBOY_GEVAL_CASE(JJ) \
-        case JJ: fn = generic_policy_evaluate_kernel<JJ>; break;
-        ROBOY_GEVAL_CASE(1) ROBOY_GEVAL_CASE(2) ROBOY_GEVAL_CASE(3) ROBOY_GEVAL_CASE(4) ROBOY_GEVAL_CASE(5)
-        ROBOY_GEVAL_CASE(6) ROBOY_GEVAL_CASE(7) ROBOY_GEVAL_CASE(8) ROBOY_GEVAL_CASE(9) ROBOY_GEVAL_CASE(10)
-        ROBOY_GEVAL_CASE(11) ROBOY_GEVAL_CASE(12) ROBOY_GEVAL_CASE(13) ROBOY_GEVAL_CASE(14) ROBOY_GEVAL_CASE(15)
+        case JJ: return launch_generic_policy(generic_policy_evaluate_kernel<JJ>, p, q, \
+                                              q.off[ROBOY_POLICY_LAYOUT_STD] - q.off[ROBOY_POLICY_LAYOUT_PI], sm_count, stream);
+        ROBOY_GENERIC_JOINT_COUNTS(ROBOY_GEVAL_CASE)
 #undef ROBOY_GEVAL_CASE
         default: return cudaErrorInvalidValue;
     }
-    cudaError_t err = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem);
-    if (err != cudaSuccess) return err;
-    fn<<<g.grid, g.block, g.smem, stream>>>(p, q);
-    return cudaGetLastError();
 }
 
 }  // namespace roboy

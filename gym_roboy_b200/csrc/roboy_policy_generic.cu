@@ -4,10 +4,10 @@
 // The shape is the MSJ kernel's (roboy_policy.cu): one launch runs T steps of [MlpPolicy forward -> Gaussian sample ->
 // clip -> RoboyEnv.step] for every env; a thread owns one env and keeps its observation row (shared memory), goal and
 // step word on chip for the T steps; both networks run in float32 FFMA2 with the weights broadcast from shared memory
-// (dense64, policy_common.cuh) and the hidden activations in a thread-private shared-memory column.  What changes with
-// the robot:
-//   * the first layer has D = 3J inputs; the observation stage has an ODD row stride (D rounded up to odd), so the 32
-//     lanes' reads of one input fall in 32 different banks;
+// (dense64, policy_common.cuh) and the hidden activations in a thread-private shared-memory column.  The frame around
+// the loop body -- shared memory, state draw, action tests, the observation stage's rows -- is policy_generic.cuh's,
+// shared with the evaluator (roboy_policy_eval.cu).  What changes with the robot:
+//   * the first layer has D = 3J inputs;
 //   * the output layer has A8 = 8 * ceil(A / 8) columns.  Its 64 inputs tanh(h2) are written back into the hidden column
 //     and it runs in groups of 8 columns, each sampled, stored, clipped and action-tested before the next, so no more
 //     than 8 outputs are ever in registers.  Every output is b3 + sum_j tanh(h2_j) * W3[j] with j ascending, the
@@ -46,17 +46,9 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_rollout_ke
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int n_warps = blockDim.x >> 5;
-    // shared memory: policy image | per warp: hidden column [64][32] | obs stage [32][S] | reduction | counters
-    const uint32_t img_floats = q.off[ROBOY_POLICY_LAYOUT_FLOATS];
-    float *img = smem;
-    float *hs = smem + img_floats + warp * (kGHid * 32) + lane;
-    float *stage = smem + img_floats + n_warps * (kGHid * 32) + warp * (32 * S);
-    double *s_red = reinterpret_cast<double *>(smem + img_floats + n_warps * (kGHid * 32 + 32 * S));
-    unsigned int *s_cnt = reinterpret_cast<unsigned int *>(s_red + n_warps);
-    for (uint32_t i = threadIdx.x; i < img_floats / 4; i += blockDim.x)
-        reinterpret_cast<float4 *>(img)[i] = reinterpret_cast<const float4 *>(q.image)[i];
-    if (threadIdx.x < kCntWords) s_cnt[threadIdx.x] = 0;
-    __syncthreads();
+    const GPolicySmem m = g_policy_smem<J>(smem, q.off[ROBOY_POLICY_LAYOUT_FLOATS]);   // the whole image
+    g_policy_smem_fill(m, q.image, q.off[ROBOY_POLICY_LAYOUT_FLOATS]);
+    const float *img = m.image;
 
     const uint64_t t_first = counter_begin(p.cc);
     const uint32_t n_end = (uint32_t)p.e_end, n_envs = (uint32_t)p.n;
@@ -68,7 +60,7 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_rollout_ke
     const float lognorm = img[q.off[ROBOY_POLICY_LAYOUT_LOGNORM]];
     const bool fastdiv = r.fastdiv != 0;   // the step kernel's choice (launch_generic_step)
     const bool act_vec = (A & 3) == 0;   // rows of actions / noise are 16-byte aligned (the buffers are)
-    float *row = stage + lane * S;
+    float *row = m.stage + lane * S;
     float sum_reward = 0.0f;
 
     for (uint32_t chunk = blockIdx.x * n_warps + warp; chunk < n_chunks; chunk += warp_stride) {
@@ -88,22 +80,22 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_rollout_ke
 
         for (uint32_t tt = 0;; ++tt) {
             // ---- value network on obs[tt] (also the bootstrap value at tt == T) ----
-            mlp_hidden<D>(vf_net, q.off, row, hs);
+            mlp_hidden<D>(vf_net, q.off, row, m.hs);
             {
                 float v[8];
-                mlp_out8(vf_net + q.off[ROBOY_POLICY_LAYOUT_W3], vf_net + q.off[ROBOY_POLICY_LAYOUT_VF_B3], 8, 0, hs, v);
+                mlp_out8(vf_net + q.off[ROBOY_POLICY_LAYOUT_W3], vf_net + q.off[ROBOY_POLICY_LAYOUT_VF_B3], 8, 0, m.hs, v);
                 if (live) q.values[(size_t)tt * n + env] = v[0];
             }
             if (tt == q.T) break;
             // ---- policy network, 8 output columns at a time: mean -> a = mean + std * z -> clip -> action tests ----
-            mlp_hidden<D>(pi_net, q.off, row, hs);
+            mlp_hidden<D>(pi_net, q.off, row, m.hs);
             const uint64_t t = t_first + tt;
             const size_t slot = (size_t)tt * n + env;
             float zz = 0.0f;
             bool act_ok = true, hold = live;
             for (int c = 0; c < A8 / 8; ++c) {
                 float mean[8];
-                mlp_out8(pi_net + q.off[ROBOY_POLICY_LAYOUT_W3], pi_net + q.off[ROBOY_POLICY_LAYOUT_PI_B3], A8, c, hs, mean);
+                mlp_out8(pi_net + q.off[ROBOY_POLICY_LAYOUT_W3], pi_net + q.off[ROBOY_POLICY_LAYOUT_PI_B3], A8, c, m.hs, mean);
                 const uint4 r0 = philox_draw(gid, t, kStreamNoise, q.noise_keys, 2 * c);
                 const uint4 r1 = philox_draw(gid, t, kStreamNoise, q.noise_keys, 2 * c + 1);
                 const float2 z01 = box_muller(r0.x, r0.y), z23 = box_muller(r0.z, r0.w);
@@ -115,11 +107,8 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_rollout_ke
                     const int k = 8 * c + i;
                     u[i] = fmaf(sd[k], z[i], mean[i]);
                     if (k < A) {
-                        const float cl = fminf(fmaxf(u[i], -1.0f), 1.0f);
-                        const float a = (u[i] != u[i]) ? u[i] : cl;   // a NaN stays a NaN (and fails the assert)
                         zz = fmaf(z[i], z[i], zz);
-                        act_ok = act_ok && (a >= -1.0f && a <= 1.0f);                      // roboy_env.py:52
-                        hold = hold && (a >= r.hold_lo[k] && a <= r.hold_hi[k]);           // simulation_client.py:38
+                        g_clip_test(r, k, u[i], act_ok, hold);
                     }
                 }
                 if (live) {
@@ -147,29 +136,15 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_rollout_ke
 
             // ---- RoboyEnv.step on the clipped action: the generic step kernel's per-env body ----
             float qs[JM], qds[JM];
-#pragma unroll
-            for (int k = 0; k < JM; ++k) qs[k] = qds[k] = 0.0f;
-            if (live) {
-                DrawCursor cur;
-                cur.block = 0xffffffffu;
-#pragma unroll
-                for (int k = 0; k < JM; ++k) qs[k] = g_draw_value(r, p.keys, gid, t, cur, k, k);
-#pragma unroll
-                for (int k = 0; k < JM; ++k) qds[k] = g_draw_value(r, p.keys, gid, t, cur, J + k, k);
-            }
-            const bool done = generic_env_step<JM>(p, fastdiv, live, hold, act_ok, qs, qds, g, sf, gid, t, env, n_envs, s_cnt,
-                                                   eplen_counter(s_cnt), sum_reward, [&](uint32_t word, float rf, bool d, bool) {
+            g_draw_step_state<JM>(r, p.keys, live, gid, t, qs, qds);
+            const bool done = generic_env_step<JM>(p, fastdiv, live, hold, act_ok, qs, qds, g, sf, gid, t, env, n_envs, m.s_cnt,
+                                                   eplen_counter(m.s_cnt), sum_reward, [&](uint32_t word, float rf, bool d, bool) {
                                                        sf = word;
                                                        p.reward[slot] = rf;
                                                        p.done[slot] = (uint8_t)d;
                                                    });
             // ---- obs[tt + 1] = [q, qd, goal] into the stage, then the chunk's 32 rows out coalesced ----
-#pragma unroll
-            for (int k = 0; k < JM; ++k) {
-                row[k] = qs[k];
-                row[J + k] = qds[k];
-                row[2 * J + k] = g[k];
-            }
+            g_stage_obs<JM>(row, qs, qds, g);
             if (done) {   // the goal of the next step (done without auto-reset: the observation above shows the old one)
 #pragma unroll
                 for (int k = 0; k < JM; ++k) g[k] = p.goal[(size_t)k * n + env];
@@ -183,27 +158,27 @@ __global__ void __launch_bounds__(kGPolicyMaxBlock, 1) generic_policy_rollout_ke
 #pragma unroll
                     for (int c = 0; c < 4; ++c) {
                         const int i = 4 * i4 + c;
-                        v[c] = stage[(i / D) * S + i % D];
+                        v[c] = m.stage[(i / D) * S + i % D];
                     }
                     dst4[i4] = make_float4(v[0], v[1], v[2], v[3]);
                 }
             } else {
                 const uint32_t rows = full ? 32u : n_end - base;
-                for (uint32_t i = lane; i < rows * D; i += 32) dst[i] = stage[(i / D) * S + i % D];
+                for (uint32_t i = lane; i < rows * D; i += 32) dst[i] = m.stage[(i / D) * S + i % D];
             }
             __syncwarp();
         }
         if (live) p.step_flags[env] = sf;
     }
 
-    policy_stats_tail(p, q.T, t_first, sum_reward, s_red, s_cnt);
+    policy_stats_tail(p, q.T, t_first, sum_reward, m.s_red, m.s_cnt);
 }
 
 PolicyGeom generic_policy_geometry(int J, uint32_t image_floats, uint64_t n_envs, int sm_count) {
     PolicyGeom g;
     g.envs_per_thread = 1;
-    const int per_warp = (int)sizeof(float) * (kGHid * 32 + 32 * g_stage_stride(J)) + (int)sizeof(double);
-    const int fixed = (int)sizeof(float) * (int)image_floats + (int)sizeof(unsigned int) * kCntWords;
+    const int fixed = g_policy_smem_bytes(J, image_floats, 0);
+    const int per_warp = g_policy_smem_bytes(J, image_floats, 1) - fixed;
     int max_warps = (kGPolicySmemBudget - fixed) / per_warp;
     if (max_warps > kGPolicyMaxBlock / 32) max_warps = kGPolicyMaxBlock / 32;
     const uint64_t n_chunks = (n_envs + 31) / 32;
@@ -212,27 +187,19 @@ PolicyGeom generic_policy_geometry(int J, uint32_t image_floats, uint64_t n_envs
     uint64_t wpb = (n_chunks + g.grid - 1) / g.grid;
     if (wpb > (uint64_t)max_warps) wpb = (uint64_t)max_warps;
     g.block = (int)wpb * 32;
-    g.smem = fixed + (int)wpb * per_warp;
+    g.smem = g_policy_smem_bytes(J, image_floats, (int)wpb);
     return g;
 }
 
 cudaError_t launch_generic_policy_rollout(const GStepParams &p, const GPolicyParams &q, int sm_count, cudaStream_t stream) {
     if (p.e_end <= p.e_begin) return cudaSuccess;
-    const PolicyGeom g = generic_policy_geometry(p.r.J, q.off[ROBOY_POLICY_LAYOUT_FLOATS], p.e_end, sm_count);
-    void (*fn)(const GStepParams, const GPolicyParams) = nullptr;
     switch (p.r.J) {
 #define ROBOY_GPOLICY_CASE(JJ) \
-        case JJ: fn = generic_policy_rollout_kernel<JJ>; break;
-        ROBOY_GPOLICY_CASE(1) ROBOY_GPOLICY_CASE(2) ROBOY_GPOLICY_CASE(3) ROBOY_GPOLICY_CASE(4) ROBOY_GPOLICY_CASE(5)
-        ROBOY_GPOLICY_CASE(6) ROBOY_GPOLICY_CASE(7) ROBOY_GPOLICY_CASE(8) ROBOY_GPOLICY_CASE(9) ROBOY_GPOLICY_CASE(10)
-        ROBOY_GPOLICY_CASE(11) ROBOY_GPOLICY_CASE(12) ROBOY_GPOLICY_CASE(13) ROBOY_GPOLICY_CASE(14) ROBOY_GPOLICY_CASE(15)
+        case JJ: return launch_generic_policy(generic_policy_rollout_kernel<JJ>, p, q, q.off[ROBOY_POLICY_LAYOUT_FLOATS], sm_count, stream);
+        ROBOY_GENERIC_JOINT_COUNTS(ROBOY_GPOLICY_CASE)
 #undef ROBOY_GPOLICY_CASE
         default: return cudaErrorInvalidValue;
     }
-    cudaError_t err = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem);
-    if (err != cudaSuccess) return err;
-    fn<<<g.grid, g.block, g.smem, stream>>>(p, q);
-    return cudaGetLastError();
 }
 
 }  // namespace roboy
