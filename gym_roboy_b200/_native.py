@@ -27,6 +27,8 @@ POLICY_OFF_VF, POLICY_OFF_PI, POLICY_OFF_STD, POLICY_OFF_LOGNORM, POLICY_IMAGE_F
 (POLICY_LAYOUT_W1, POLICY_LAYOUT_B1, POLICY_LAYOUT_W2, POLICY_LAYOUT_B2, POLICY_LAYOUT_W3, POLICY_LAYOUT_VF_B3, POLICY_LAYOUT_PI_B3,
  POLICY_LAYOUT_VF, POLICY_LAYOUT_PI, POLICY_LAYOUT_STD, POLICY_LAYOUT_LOGNORM, POLICY_LAYOUT_FLOATS) = range(12)
 POLICY_LAYOUT_WORDS = 12
+# roboy_ppo_grad's statistics vector (ROBOY_PPO_STAT_*)
+PPO_STAT_NAMES = ("loss", "pg_loss", "vf_loss", "entropy", "approxkl", "clipfrac", "adv_mean", "adv_std", "bad_indices")
 # ... and of the tensor-core variant's image (ROBOY_TC_*): float16 element offsets, then byte offsets
 TC_K_HIDDEN = 80
 TC_OFF_W1, TC_OFF_W2, TC_OFF_W3, TC_NET_HALVES, TC_OFF_VF, TC_OFF_PI = 0, 1024, 6144, 7424, 0, 7424
@@ -114,6 +116,9 @@ SIGNATURES = {
     "roboy_policy_tc_geometry": (_int, [_vp, _int, _int, ctypes.POINTER(_int), ctypes.POINTER(_int), ctypes.POINTER(_int),
                                         ctypes.POINTER(_int)]),
     "roboy_policy_layout": (_int, [_int, _int, ctypes.POINTER(ctypes.c_uint32)]),
+    "roboy_ppo_workspace_bytes": (_int, [_int, _int, _u64, ctypes.POINTER(_u64)]),
+    "roboy_ppo_grad": (_int, [_int, _int, _vp, _u64, _vp, _u64, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, ctypes.c_float,
+                              ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _vp]),
     "roboy_policy_geometry": (_int, [_vp, _int, ctypes.POINTER(_int), ctypes.POINTER(_int), ctypes.POINTER(_int),
                                      ctypes.POINTER(_int)]),
     "roboy_launch_count": (_int, [_vp, ctypes.POINTER(_u64)]),

@@ -13,7 +13,7 @@ CSRC = os.path.join(_PKG, "csrc")
 LIB_DIR = os.path.join(_PKG, "_lib")
 LIB_PATH = os.path.join(LIB_DIR, "libroboy_b200.so")
 SOURCES = ("roboy_kernels.cu", "roboy_generic.cu", "roboy_policy.cu", "roboy_policy_tc.cu", "roboy_policy_generic.cu", "roboy_policy_eval.cu",
-           "roboy_capi.cu")
+           "roboy_ppo.cu", "roboy_capi.cu")
 HEADERS = ("roboy_kernels.cuh", "roboy_generic.cuh", "generic_env.cuh", "roboy_policy.cuh", "policy_common.cuh", "policy_generic.cuh", "step_rare.cuh", "msj_math.cuh", "philox.cuh", "dlpack_min.h", os.path.join("..", "..", "include", "roboy_b200.h"))
 
 NVCC_FLAGS = [

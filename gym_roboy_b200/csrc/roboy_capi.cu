@@ -1484,6 +1484,77 @@ int roboy_policy_layout(int dim_obs, int dim_action, uint32_t *offsets) {
     return ROBOY_OK;
 }
 
+// Bytes from dev_ptr to the end of the device allocation holding it (cuMemGetAddressRange through the runtime's
+// driver entry point: no link against libcuda).  false if dev_ptr is not in a device allocation.
+static bool allocation_room(const void *dev_ptr, uint64_t *room) {
+    typedef int (*GetRange)(unsigned long long *base, size_t *size, unsigned long long ptr);
+    static GetRange get_range = nullptr;
+    if (!get_range) {
+        void *fn = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &fn, cudaEnableDefault, &q) != cudaSuccess ||
+            q != cudaDriverEntryPointSuccess || !fn)
+            return false;
+        get_range = (GetRange)fn;
+    }
+    unsigned long long base = 0;
+    size_t size = 0;
+    if (get_range(&base, &size, (unsigned long long)(uintptr_t)dev_ptr) != 0) return false;
+    *room = base + size - (uint64_t)(uintptr_t)dev_ptr;
+    return true;
+}
+
+int roboy_ppo_workspace_bytes(int dim_obs, int dim_action, uint64_t M, uint64_t *bytes) {
+    if (!bytes) return fail(ROBOY_E_ARG, "NULL bytes");
+    uint32_t off[ROBOY_POLICY_LAYOUT_WORDS];
+    if (roboy_policy_layout(dim_obs, dim_action, off) != ROBOY_OK) return ROBOY_E_ARG;
+    if (M == 0) return fail(ROBOY_E_ARG, "the minibatch is empty (M == 0)");
+    *bytes = ppo_workspace_bytes(off[ROBOY_POLICY_LAYOUT_FLOATS], M);
+    return ROBOY_OK;
+}
+
+int roboy_ppo_grad(int dim_obs, int dim_action, const float *image_dev, uint64_t M, const int64_t *index_dev,
+                   uint64_t n_rows, const float *obs_dev, const float *actions_dev, const float *logp_dev,
+                   const float *values_dev, const float *ret_dev, float clip_range, float clip_range_vf,
+                   float ent_coef, float vf_coef, float *grad_dev, double *stats_dev, void *workspace_dev,
+                   void *stream) {
+    PpoParams p{};
+    if (roboy_policy_layout(dim_obs, dim_action, p.off) != ROBOY_OK) return ROBOY_E_ARG;
+    if (M == 0) return fail(ROBOY_E_ARG, "the minibatch is empty (M == 0)");
+    if (!image_dev || !index_dev || !obs_dev || !actions_dev || !logp_dev || !values_dev || !ret_dev || !grad_dev ||
+        !stats_dev || !workspace_dev)
+        return fail(ROBOY_E_ARG, "NULL device pointer");
+    if ((uintptr_t)image_dev & 15) return fail(ROBOY_E_ARG, "image must be 16-byte aligned");
+    if ((uintptr_t)workspace_dev & 7) return fail(ROBOY_E_ARG, "workspace must be 8-byte aligned");
+    p.P = p.off[ROBOY_POLICY_LAYOUT_FLOATS];
+    // the bytes from workspace_dev to the end of the allocation that holds it (a pool allocator's block may be larger
+    // than the caller's tensor: this catches what would run past the allocation)
+    const uint64_t need = ppo_workspace_bytes(p.P, M);
+    uint64_t room = 0;
+    if (!allocation_room(workspace_dev, &room) || room < need)
+        return fail(ROBOY_E_ARG, "the workspace holds %llu bytes; roboy_ppo_workspace_bytes asks for %llu",
+                    (unsigned long long)room, (unsigned long long)need);
+    p.J = dim_obs / 3;
+    p.A = dim_action;
+    p.M = M;
+    p.n_rows = n_rows;
+    p.image = image_dev;
+    p.index = index_dev;
+    p.obs = obs_dev;
+    p.actions = actions_dev;
+    p.logp = logp_dev;
+    p.values = values_dev;
+    p.ret = ret_dev;
+    p.clip = clip_range;
+    p.clip_vf = clip_range_vf;
+    p.ent_coef = ent_coef;
+    p.vf_coef = vf_coef;
+    p.grad = grad_dev;
+    p.stats = stats_dev;
+    CUDA_TRY(launch_ppo_grad(p, workspace_dev, (cudaStream_t)stream));
+    return ROBOY_OK;
+}
+
 int roboy_policy_geometry(roboy_env *env, int envs_per_thread, int *grid, int *block, int *smem_bytes, int *ept) {
     if (check_env(env)) return ROBOY_E_ARG;
     PolicyGeom geo;

@@ -85,4 +85,27 @@ struct GEvalParams {
 };
 cudaError_t launch_generic_policy_evaluate(const GStepParams &p, const GEvalParams &q, int sm_count, cudaStream_t stream);
 
+// PPO2 minibatch gradient (roboy_ppo.cu) for every robot: one 64-sample tile at a time per CTA of 128 threads, one CTA per
+// slot, slots = min(tiles, kPpoMaxSlots): a function of M only, so the partial sums and their order are too.
+constexpr int kPpoTile = 64, kPpoThreads = 128, kPpoMaxSlots = 1184, kPpoAdvBlocks = 256, kPpoAdvThreads = 256;
+struct PpoParams {
+    const float *__restrict__ image;           // roboy_policy_layout(3J, A) image
+    uint32_t off[ROBOY_POLICY_LAYOUT_WORDS];
+    uint32_t P;                                // off[ROBOY_POLICY_LAYOUT_FLOATS]
+    int J, A;
+    uint64_t M, n_rows;
+    const int64_t *__restrict__ index;         // [M]
+    const float *__restrict__ obs;             // [n_rows][3J]
+    const float *__restrict__ actions;         // [n_rows][A]
+    const float *__restrict__ logp, *__restrict__ values, *__restrict__ ret;   // [n_rows]
+    float clip, clip_vf, ent_coef, vf_coef;    // clip_vf < 0: no value clipping
+    float *__restrict__ grad;                  // [P]
+    double *__restrict__ stats;                // [ROBOY_PPO_STAT_COUNT]
+    double *adv_part, *stat_part;              // workspace, carved by launch_ppo_grad
+    float *grad_part;
+};
+uint32_t ppo_slots(uint64_t M);
+uint64_t ppo_workspace_bytes(uint32_t P, uint64_t M);
+cudaError_t launch_ppo_grad(PpoParams p, void *workspace, cudaStream_t stream);
+
 }  // namespace roboy

@@ -462,6 +462,55 @@ int roboy_policy_rollout_tc(roboy_env *env, uint32_t T, const float *tc_image_de
 int roboy_policy_evaluate(roboy_env *env, uint32_t T, const float *image_dev, float *obs_dev, uint32_t episodes,
                           double *returns_dev, uint32_t *lengths_dev, uint8_t *reached_dev, uint32_t *completed_dev,
                           void *stream);
+/* PPO2 update (stable-baselines 2's PPO2._train_step, as documented upstream): the clipped-surrogate loss of one minibatch
+ * and its gradient with respect to every MlpPolicy parameter, in float32, on every robot (dim_obs = 3J, J = 1..15;
+ * dim_action = A = 1..64).  Handle-free; runs on the current device, async on `stream`.
+ *  1. Samples: s = index_dev[i], i < M (64-bit row offsets into the [n_rows] buffers obs [n_rows][D], actions
+ *     [n_rows][A] (the UN-clipped samples), logp, values (the values at collection), ret).  An index outside
+ *     [0, n_rows) is counted (ROBOY_PPO_STAT_BAD_INDICES) and skipped, not read; every mean below is over the
+ *     M_valid = M - bad valid samples (zero when there are none).
+ *  2. Advantages: adv_s = ret_s - values_s (float32), normalised over the minibatch as (adv - mean) / (std + 1e-8), with
+ *     the population std; the sums are float64.
+ *  3. Policy: mean, v = the float32 MlpPolicy at obs_s; std = the image's std (exp(log_std)); z = (a - mean) / std;
+ *     logp_new = lognorm - 1/2 sum z^2; ratio = exp(logp_new - logp_old).
+ *  4. Loss: pg_loss = mean(max(-adv ratio, -adv clip(ratio, 1 - clip_range, 1 + clip_range)));
+ *     vf_loss = 1/2 mean(max((v - R)^2, (v_clip - R)^2)), v_clip = v_old + clip(v - v_old, -clip_range_vf, clip_range_vf),
+ *     or 1/2 mean((v - R)^2) when clip_range_vf < 0;  entropy = sum_k (log_std_k + 1/2 log(2 pi e));
+ *     loss = pg_loss - ent_coef entropy + vf_coef vf_loss.
+ *  5. Gradients follow TF's rules: maximum(x, y) passes the gradient to x where x >= y, clip_by_value passes it inside
+ *     the closed range; the advantages and the old values are constants.
+ *  6. grad_dev: d loss / d parameter in the layout of image_dev (roboy_policy_layout(dim_obs, dim_action)); the std slots
+ *     hold d loss / d log_std; padded columns, the padded std slots and the lognorm slot are 0.
+ *  7. stats_dev double[ROBOY_PPO_STAT_COUNT]; approxkl = 1/2 mean((logp_new - logp_old)^2), clipfrac = mean(|ratio - 1| >
+ *     clip_range).
+ *  8. Determinism: the result depends only on the inputs (not on the device, the stream or a CUDA-graph replay), bit
+ *     for bit: every partial sum has a fixed place and order.
+ *  9. workspace_dev: at least roboy_ppo_workspace_bytes(dim_obs, dim_action, M) bytes, 8-byte aligned.  The caller
+ *     must provide that size: the call sees no buffer size, only the device allocation that holds workspace_dev.
+ * 10. Refusals (ROBOY_E_ARG): dims outside the layout's range, M == 0, a NULL pointer, an image not 16-byte aligned, a
+ *     workspace not 8-byte aligned, not in device memory, or with fewer bytes than that between workspace_dev and the
+ *     end of its device allocation (cuMemGetAddressRange).  A buffer carved from a larger allocation (a pool
+ *     allocator's block) is checked against the end of that allocation, not against the buffer's own end.
+ * Algorithmic FMAs per sample (hidden width 64): 256 D + 24,576 + 192 (A + 1). */
+enum {
+    ROBOY_PPO_STAT_LOSS = 0,
+    ROBOY_PPO_STAT_PG_LOSS = 1,
+    ROBOY_PPO_STAT_VF_LOSS = 2,
+    ROBOY_PPO_STAT_ENTROPY = 3,
+    ROBOY_PPO_STAT_APPROXKL = 4,
+    ROBOY_PPO_STAT_CLIPFRAC = 5,
+    ROBOY_PPO_STAT_ADV_MEAN = 6,     /* of the raw advantages ret - values over the valid samples */
+    ROBOY_PPO_STAT_ADV_STD = 7,      /* population std of the same */
+    ROBOY_PPO_STAT_BAD_INDICES = 8,  /* indices outside [0, n_rows) */
+    ROBOY_PPO_STAT_COUNT = 9
+};
+int roboy_ppo_workspace_bytes(int dim_obs, int dim_action, uint64_t M, uint64_t *bytes);
+int roboy_ppo_grad(int dim_obs, int dim_action, const float *image_dev, uint64_t M, const int64_t *index_dev,
+                   uint64_t n_rows, const float *obs_dev, const float *actions_dev, const float *logp_dev,
+                   const float *values_dev, const float *ret_dev, float clip_range, float clip_range_vf,
+                   float ent_coef, float vf_coef, float *grad_dev, double *stats_dev, void *workspace_dev,
+                   void *stream);
+
 /* Launch geometry roboy_policy_rollout uses for this handle (bench.py / tests); ept = envs per thread.  Refuses the
  * envs_per_thread values roboy_policy_rollout refuses (robots other than MSJ: 0 or 1). */
 int roboy_policy_geometry(roboy_env *env, int envs_per_thread, int *grid, int *block, int *smem_bytes, int *ept);
